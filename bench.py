@@ -8,14 +8,14 @@ D=48/32/8, batch 1 (BASELINE.json configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]        # this implementation
     python bench.py --impl reference ...                         # the reference's own DepthNet on the host cores
+    python bench.py ... --dump-outputs DIR                       # also write the last timed step's outputs as DIR/*.npy
 
 One process per GPU (torchrun for N>1); reference views are independent, so ranks
 share nothing on the data path and the scaling is weak (K views per rank).
 Prints ONE JSON line on rank 0.
 
 Legs of the main line (all on the same box, same run):
-  value          K-step batches of the hot path, inputs resident in HBM, repeated until >= 1 s of device time; the
-                 MEDIAN batch (max over ranks per batch) is reported
+  value          exactly K steps of the hot path, inputs resident in HBM, timed as one batch (max over ranks)
   e2e            the same through HotPathRunner.submit_host/collect from pinned host buffers
   roofline(s)    per-kernel-class device time (CUDA events around every C-ABI call) against SURVEY.md 8d's algorithmic
                  bytes / flops
@@ -50,7 +50,8 @@ UNIT = "views/s"
 def parse(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=400,
+                    help="timed steps, run as one batch (the default covers about 1 s of device time on a B200)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--precision", default="fp16", choices=["fp16", "bf16", "fp32"],
@@ -66,13 +67,20 @@ def parse(argv=None):
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-incumbent", action="store_true", help="skip the reference-on-this-GPU legs")
     ap.add_argument("--no-extras", action="store_true", help="skip the fp32 / T&T / training / full-forward legs")
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="device time the timed region must cover (batches are repeated)")
+    ap.add_argument("--min-seconds", type=float, default=1.0,
+                    help="device time the e2e and Tanks-and-Temples legs must cover (their batches are repeated)")
     ap.add_argument("--budget-s", type=float, default=150.0, help="--impl reference: wall-clock budget of the timed passes")
     ap.add_argument("--detail", action="store_true", help="print a per-layer device-time table to stderr")
     ap.add_argument("--no-graph", action="store_true", help="launch kernels eagerly instead of replaying a CUDA graph")
     ap.add_argument("--fuse-prob-head", action="store_true", help="run CostRegNet's last layer fused with the head (one launch)")
     ap.add_argument("--inflight", type=int, default=4, help="independent views in flight on separate streams (graph mode)")
-    return ap.parse_args(argv)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the per-stage outputs of the last one (rank 0) as DIR/stage<s>_<key>.npy "
+                         "in float32; see dump_outputs()")
+    args = ap.parse_args(argv)
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this implementation's timed path; it does not apply to --impl reference")
+    return args
 
 
 def peaks():
@@ -329,6 +337,26 @@ def timed_batches(run_views, steps, min_seconds, barrier, dev, max_reps=40):
     return statistics.median(times), times, len(times)
 
 
+DUMP_BYTES = 60_000_000
+
+
+def dump_outputs(out_dir, outs, seed=0):
+    """Write one step's per-stage output dicts (what HotPathRunner.run_device returns) as out_dir/stage<s>_<key>.npy in
+    float32, so that two builds run with the same arguments can be compared array for array.  The arrays share
+    DUMP_BYTES equally: one larger than its share is stored as a 1-D sample of its flattened values at fixed indices (a
+    seeded random subset, sorted, that depends only on the array's size); the others keep their shape."""
+    import numpy as np
+    arrays = {f"stage{s + 1}_{k}": v for s, out in enumerate(outs) for k, v in out.items()}
+    cap = DUMP_BYTES // 4 // len(arrays)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().float()
+        if a.numel() > cap:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(seed))[:cap].sort().values
+            a = a.flatten()[idx.to(a.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
+
+
 def numa_pin(local_rank: int) -> str:
     """Bind this process to the CPUs of the NUMA node its GPU hangs off, BEFORE the pinned host buffers are allocated
     (first touch places them on that node), so that 8 ranks do not all stream their uploads out of node 0."""
@@ -572,15 +600,18 @@ def run_ours(args):
 
     def make_run_views(rn, stages):
         pipe = None if args.no_graph else ViewPipeline(rn, shifted_sets(stages, inflight))
+        last = [None]
 
         def run_views(n):
             if pipe is None:
                 for _ in range(n):
-                    rn.run_device(stages)
+                    last[0] = rn.run_device(stages)
             else:
                 pipe.fork()
                 pipe.submit(n)
                 pipe.join()
+                last[0] = pipe.last_outputs()
+        run_views.last_outputs = lambda: last[0]
         return run_views
 
     run_views = make_run_views(runner, dev_stages)
@@ -589,8 +620,10 @@ def run_ours(args):
     barrier()
     if rank == 0:
         sampler.start()
-    batch_ms, all_ms, reps = timed_batches(run_views, steps, args.min_seconds, barrier, dev)
+    batch_ms, all_ms, _ = timed_batches(run_views, steps, 0.0, barrier, dev, max_reps=1)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, run_views.last_outputs())
     # kernels per step = C-ABI launches of one eager pass (graph replays do not pass through the C ABI)
     n0 = _lib.launch_count()
     runner.run_device(dev_stages)
@@ -803,8 +836,8 @@ def run_ours(args):
                 "dtype": args.precision, "data": "synthetic",
                 "config": config_of(args, {"parallelism": f"views sharded x{world}, no data-path collective",
                                            "launch": "eager" if args.no_graph else f"cuda-graph replay of the 3-stage step, {inflight} independent views in flight on {inflight} streams",
-                                           "timing": f"median of {reps} batches of {steps} steps (each batch bracketed by barrier + synchronize, CUDA events, max over ranks); "
-                                                     f"{sum(all_ms) / 1e3:.2f} s of device time in total"}),
+                                           "timing": f"one batch of {steps} steps (bracketed by barrier + synchronize, CUDA events, max over ranks); "
+                                                     f"{sum(all_ms) / 1e3:.2f} s of device time"}),
                 "batches_ms": all_ms, "clocks": clocks, "e2e": e2e, "gpu_launches": int(launches), "roofline": roof,
                 "rooflines": rooflines, "kernels": kernels, "cpu_baseline": cpu, "incumbent_gpu": incumbent, "extras": extras}
         print(json.dumps(line), flush=True)

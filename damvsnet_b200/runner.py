@@ -325,6 +325,10 @@ class ViewPipeline:
             ev.record(s)
             cur.wait_event(ev)
 
+    def last_outputs(self) -> List[Dict[str, torch.Tensor]]:
+        """The output buffers of the view submitted last (complete once the current stream has passed join())."""
+        return self.outputs[(self._next - 1) % len(self.graphs)]
+
 
 class HostTicket:
     def __init__(self, host, event):

@@ -1,7 +1,7 @@
 """Group-wise correlation cost volume (NOT in the reference: BASELINE.json north star / configs[4]).
 
-CPU: the own-restatement oracle (oracle/gwc_oracle.py) against a direct formulation built on F.grid_sample, and -- when
-the reference code is available -- on the reference's own ``homo_warping``.  GPU (-m gpu): csrc/warp_gwc.cu against that
+CPU: the own-restatement oracle (oracle/gwc_oracle.py) against a direct formulation built on F.grid_sample, and on the
+stored outputs of the reference's own ``homo_warping``.  GPU (-m gpu): csrc/warp_gwc.cu against that
 oracle for every supported (C, G), both feature widths, ragged extents, [B,D] and [B,D,H,W] hypotheses, and through
 CostRegNet + head as a DepthNet mode.
 """
@@ -10,7 +10,7 @@ import torch
 import torch.nn.functional as F
 
 from oracle import damvs_oracle as O
-from oracle import gwc_oracle, ref_loader
+from oracle import gwc_oracle
 
 CASES = [(8, 4), (8, 8), (16, 4), (16, 8), (16, 16), (32, 4), (32, 8), (32, 16), (32, 32)]
 
@@ -38,20 +38,21 @@ def test_gwc_oracle_matches_a_direct_grid_sample_formulation():
     assert got.shape == (2, 8, 6, 16, 24)          # stage 2 of a 32x48 image
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference code neither staged nor mounted")
 def test_gwc_oracle_uses_the_references_warp():
-    import warnings
-    _, rm = ref_loader.load()
-    feats, pm, dv = _inputs(0, 1, 3, 32, 32, 5, 4, 32)
-    got = gwc_oracle.groupwise_correlation(feats, pm, dv, 4)
-    projs = [O.compose_projection(p) for p in torch.unbind(pm, 1)]
-    want = torch.zeros_like(got)
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        for src, sp in zip(feats[1:], projs[1:]):
-            warped = rm.homo_warping(src, sp, projs[0], dv)
-            want += (feats[0].unsqueeze(2) * warped).view(1, 4, 8, 5, 8, 8).mean(2)     # stage 1 of a 32x32 image is 8x8
-    torch.testing.assert_close(got, want / 2, rtol=1e-4, atol=1e-5)
+    """Against the reference's own homo_warping outputs stored in tests/golden/homo_warping.npz (one source view, [B,D,H,W]
+    and [B,D] hypotheses).  The stored projections are already composed, so they enter as extrinsics with identity
+    intrinsics."""
+    from tests import golden_io
+    g = golden_io.load_homo()
+    src = g["src"]
+    b, c, h, w = src.shape
+    eye = torch.eye(4).expand(b, 4, 4)
+    pm = torch.stack([torch.stack([g["ref_proj"], eye], 1), torch.stack([g["src_proj"], eye], 1)], 1)     # [B,2,2,4,4]
+    ref = torch.randn(b, c, h, w, generator=torch.Generator().manual_seed(4))
+    for dv, warped in ((g["dv4"], g["out4"]), (g["dv2"], g["out2"])):
+        got = gwc_oracle.groupwise_correlation([ref, src], pm, dv, 4)
+        want = (ref.unsqueeze(2) * warped).view(b, 4, c // 4, dv.shape[1], h, w).mean(2)
+        torch.testing.assert_close(got, want, rtol=1e-4, atol=1e-5)
 
 
 # ------------------------------------------------------------------------------------------------ GPU
