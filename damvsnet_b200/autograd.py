@@ -53,7 +53,7 @@ class ConvBlockFn(torch.autograd.Function):
     packed-weight caches, BatchNorm buffers)."""
 
     @staticmethod
-    def forward(ctx, x, skip, weight, gamma, beta, blk):
+    def forward(ctx, x, skip, weight, gamma, beta, bias, blk):
         cin, cout, stride, tr = blk.in_channels, blk.out_channels, blk.stride, blk.transposed
         impl = ops.conv_impl_for(cin, cout, stride, tr)
         y = ops.conv3d(G8Volume(x), blk.packed_weight(impl), None, None, cout, stride, tr, False, None, x.dtype, False,
@@ -71,7 +71,7 @@ class ConvBlockFn(torch.autograd.Function):
             mean = torch.zeros(cout, dtype=torch.float32, device=x.device)
             rstd = torch.ones_like(mean)
             scale = torch.ones_like(mean)
-            shift = blk.conv.bias.detach().float() if blk.conv.bias is not None else torch.zeros_like(mean)
+            shift = bias.detach().float() if bias is not None else torch.zeros_like(mean)
         out = ops_train.bn_apply(y, scale, shift, skip, blk.relu)
         ctx.blk, ctx.batch, ctx.has_skip = blk, batch, skip is not None
         ctx.save_for_backward(x, y, scale, shift, mean, rstd)
@@ -91,12 +91,16 @@ class ConvBlockFn(torch.autograd.Function):
         else:
             g_y, sums = ops_train.bn_bwd(g_out, y, scale, shift, scale, None, None, blk.relu, True, True)
             _, _, _, dgamma, dbeta = ops_train.bn_bwd_coeffs(sums, scale, mean, rstd, m, False)
-        g_x = g_w = g_gamma = g_beta = None
+        g_x = g_w = g_gamma = g_beta = g_bias = None
         if ctx.needs_input_grad[0]:
             a_stride, a_tr = (1, False) if (stride == 1 and not tr) else ((2, False) if tr else (2, True))
             impl = ops.conv_impl_for(cout, cin, a_stride, a_tr)
             g_x = ops.conv3d(G8Volume(g_y), blk.packed_adjoint(impl), None, None, cin, a_stride, a_tr, False, None, g_y.dtype,
                              False, impl).data
+            if g_x.shape != x.shape:
+                # the adjoint of a stride-2 conv over an odd extent is a transposed conv one plane longer than x (2 * ceil(n/2)
+                # planes); the extra plane pairs with no input voxel, so the data gradient is its crop
+                g_x = g_x[:, :, :x.shape[2], :x.shape[3], :x.shape[4]].contiguous()
         if ctx.needs_input_grad[2]:
             g_w = ops_train.conv3d_wgrad(x, g_y, cin, cout, stride, tr)
         if blk.bn is not None:
@@ -104,8 +108,10 @@ class ConvBlockFn(torch.autograd.Function):
                 g_gamma = dgamma
             if ctx.needs_input_grad[4]:
                 g_beta = dbeta
+        elif ctx.needs_input_grad[5]:
+            g_bias = dbeta               # without BatchNorm the conv bias is the shift: its gradient is the channel sum of g_z
         g_skip = g_out if (ctx.has_skip and ctx.needs_input_grad[1]) else None
-        return g_x, g_skip, g_w, g_gamma, g_beta, None
+        return g_x, g_skip, g_w, g_gamma, g_beta, g_bias, None
 
 
 class ProbConvFn(torch.autograd.Function):
@@ -152,6 +158,51 @@ class HeadFn(torch.autograd.Function):
         g_logits, g_hyp = ops_train.softmax_regress_bwd(prob, dv, depth, g_depth, g_var, g_prob,
                                                         want_hyp_grad=ctx.needs_input_grad[1])
         return g_logits, g_hyp
+
+
+class DepthRegressionFn(torch.autograd.Function):
+    """depth = sum_d p * depth_values (native kernel); backward g_p = g * dv, g_dv = g * p (D planes of tensor ops)."""
+
+    @staticmethod
+    def forward(ctx, p, depth_values):
+        ctx.save_for_backward(p, depth_values)
+        return ops.depth_regression(p, depth_values)
+
+    @staticmethod
+    def backward(ctx, g):
+        p, dv = ctx.saved_tensors
+        g = g.unsqueeze(1)
+        dv4 = dv if dv.dim() == 4 else dv.view(*dv.shape, 1, 1)
+        g_p = g * dv4 if ctx.needs_input_grad[0] else None
+        g_dv = None
+        if ctx.needs_input_grad[1]:
+            g_dv = g * p if dv.dim() == 4 else (g * p).sum(dim=(2, 3))
+        return g_p, g_dv
+
+
+class NcdhwToG8Fn(torch.autograd.Function):
+    """[B,C,D,H,W] fp32 -> G8 data tensor of `dtype` (layout kernel); the backward is the opposite layout kernel."""
+
+    @staticmethod
+    def forward(ctx, x, dtype):
+        return G8Volume.from_ncdhw(x, dtype).data
+
+    @staticmethod
+    def backward(ctx, g):
+        return G8Volume(g.contiguous()).to_ncdhw(), None
+
+
+class G8ToNcdhwFn(torch.autograd.Function):
+    """G8 data tensor -> [B,C,D,H,W] fp32 (layout kernel); the backward is the opposite layout kernel."""
+
+    @staticmethod
+    def forward(ctx, data):
+        ctx.dtype = data.dtype
+        return G8Volume(data).to_ncdhw()
+
+    @staticmethod
+    def backward(ctx, g):
+        return G8Volume.from_ncdhw(g.contiguous().float(), ctx.dtype).data
 
 
 class NhwcFn(torch.autograd.Function):

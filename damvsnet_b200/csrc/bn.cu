@@ -5,7 +5,7 @@
 // (+ skip) pass and the backward of that pass are the HBM-streaming kernels below.  All of them work on G8
 // volumes [B][C/8][D][H][W][8] (bf16 or fp32), one thread per (voxel, 8-channel group), 16/32-byte accesses.
 //
-//   bn_stats_kernel    sums[c] += {sum y, sum y^2} over (B,D,H,W)        (fp32 partials, fp64 atomics)
+//   bn_stats_kernel    sums[c] += {sum y, sum y^2} over (B,D,H,W)        (fp32 partials around a pivot, fp64 atomics)
 //   bn_apply_kernel    out = skip + act(y * scale[c] + shift[c])
 //   bn_bwd_kernel      g_z = g_out * [act active];  sums[c] += {sum g_z, sum g_z*y};
 //                      g_y = k1[c] * g_z + k2[c] * y + k3[c]
@@ -26,13 +26,17 @@ __global__ void __launch_bounds__(256) bn_stats_kernel(const T* __restrict__ y, 
 #pragma unroll
   for (int j = 0; j < 8; ++j) a[j] = q[j] = 0.f;
   const T* base = y + (size_t)bg * V * 8;
+  // fp32 partials of (y - p) around a per-block pivot p (the block's first voxel), un-shifted in fp64: raw fp32 sums of
+  // y and y^2 lose the variance to cancellation once |mean| >> std (relative error ~ (mean/std)^2 * 2^-24)
+  const long long vb = (long long)blockIdx.x * blockDim.x * kStatVox;
+  const F8 pv = load8(base + vb * 8);
 #pragma unroll 4
   for (int k = 0; k < kStatVox; ++k) {
     const long long v = v0 + (long long)k * blockDim.x;
     if (v < V) {
       const F8 r = load8(base + v * 8);
 #pragma unroll
-      for (int j = 0; j < 8; ++j) { a[j] += r.v[j]; q[j] = fmaf(r.v[j], r.v[j], q[j]); }
+      for (int j = 0; j < 8; ++j) { const float d = r.v[j] - pv.v[j]; a[j] += d; q[j] = fmaf(d, d, q[j]); }
     }
   }
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -46,11 +50,13 @@ __global__ void __launch_bounds__(256) bn_stats_kernel(const T* __restrict__ y, 
     if (lane == 0) { s_part[warp][j][0] = a[j]; s_part[warp][j][1] = q[j]; }
   }
   __syncthreads();
-  if (threadIdx.x < 16) {
-    const int j = threadIdx.x >> 1, w = threadIdx.x & 1;
-    double s = 0.0;
-    for (int k = 0; k < 8; ++k) s += (double)s_part[k][j][w];
-    atomicAdd(sums + (g * 8 + j) * 2 + w, s);
+  if (threadIdx.x < 8) {
+    const int j = threadIdx.x;
+    double s1 = 0.0, s2 = 0.0;
+    for (int k = 0; k < 8; ++k) { s1 += (double)s_part[k][j][0]; s2 += (double)s_part[k][j][1]; }
+    const double p = pv.v[j], n = (double)min((long long)blockDim.x * kStatVox, V - vb);
+    atomicAdd(sums + (g * 8 + j) * 2, s1 + n * p);
+    atomicAdd(sums + (g * 8 + j) * 2 + 1, s2 + p * (2.0 * s1 + n * p));
   }
 }
 
@@ -96,6 +102,14 @@ __global__ void __launch_bounds__(256) bn_bwd_kernel(const T* __restrict__ g_out
     c3[j] = k3 ? __ldg(k3 + g * 8 + j) : 0.f;
   }
   const size_t base = (size_t)bg * V * 8;
+  // sum g_z * y accumulated as sum g_z * (y - p) + p * sum g_z (pivot p as in bn_stats_kernel), so that the backward's
+  // sum g_z y - mean * sum g_z cancels in fp64 rather than in the fp32 partials
+  float pv[8];
+  {
+    const F8 r = load8(y + base + (size_t)blockIdx.x * blockDim.x * kStatVox * 8);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) pv[j] = r.v[j];
+  }
 #pragma unroll 2
   for (int k = 0; k < kStatVox; ++k) {
     const long long v = v0 + (long long)k * blockDim.x;
@@ -108,7 +122,7 @@ __global__ void __launch_bounds__(256) bn_bwd_kernel(const T* __restrict__ g_out
         const bool on = !relu || fmaf(yy.v[j], sc[j], sh[j]) > 0.f;
         const float gz = on ? go.v[j] : 0.f;
         a[j] += gz;
-        q[j] = fmaf(gz, yy.v[j], q[j]);
+        q[j] = fmaf(gz, yy.v[j] - pv[j], q[j]);
         r.v[j] = fmaf(c1[j], gz, fmaf(c2[j], yy.v[j], c3[j]));
       }
       if (g_y) store8(g_y + off, r);
@@ -126,11 +140,12 @@ __global__ void __launch_bounds__(256) bn_bwd_kernel(const T* __restrict__ g_out
       if (lane == 0) { s_part[warp][j][0] = a[j]; s_part[warp][j][1] = q[j]; }
     }
     __syncthreads();
-    if (threadIdx.x < 16) {
-      const int j = threadIdx.x >> 1, w = threadIdx.x & 1;
-      double s = 0.0;
-      for (int k = 0; k < 8; ++k) s += (double)s_part[k][j][w];
-      atomicAdd(sums + (g * 8 + j) * 2 + w, s);
+    if (threadIdx.x < 8) {
+      const int j = threadIdx.x;
+      double s1 = 0.0, s2 = 0.0;
+      for (int k = 0; k < 8; ++k) { s1 += (double)s_part[k][j][0]; s2 += (double)s_part[k][j][1]; }
+      atomicAdd(sums + (g * 8 + j) * 2, s1);
+      atomicAdd(sums + (g * 8 + j) * 2 + 1, s2 + (double)pv[j] * s1);
     }
   }
 }

@@ -79,7 +79,7 @@ __device__ __forceinline__ void group_barrier(int g) {   // constant ids: a regi
 }
 
 // exp(x), x <= 0, argument clamped at -80: keeps e and e / s out of the denormal slow paths (see head.cu)
-__device__ __forceinline__ float exp_clamped_p(float x) { return expf(fmaxf(x, -80.f)); }
+__device__ __forceinline__ float exp_clamped_p(float x) { return expf(x < -80.f ? -80.f : x); }   // NaN propagates (head.cu)
 
 // HEAD = true fuses the softmax / regression / confidence / variance head (head.cu; reference models/cas_mvsnet.py:105-124)
 // into the epilogue: the CTA owns all D output planes of its 6 x 30 pixels, so the logits go to shared memory ([D][8][32]

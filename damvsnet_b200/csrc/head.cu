@@ -26,7 +26,9 @@ constexpr int kHeadPix = 128;
 // denormals, and both expf and the IEEE division p = e / s drop into their slow paths (ncu, stage 2 of the benchmark:
 // 162 warp instructions per (warp, hypothesis), 111 us for 182 MB).  exp(-80) = 1.8e-35 keeps e and e / s (s <= D) in the
 // normal range; the probabilities it replaces are < 1.8e-35 in the reference too, far below one fp32 ulp of any output.
-__device__ __forceinline__ float exp_clamped(float x) { return expf(fmaxf(x, -80.f)); }
+// The clamp is a compare, not fmaxf: fmaxf(NaN, -80) is -80, which would turn a NaN logit into a finite probability
+// and hide a diverged training step behind plausible depth / confidence / variance.
+__device__ __forceinline__ float exp_clamped(float x) { return expf(x < -80.f ? -80.f : x); }
 
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc));

@@ -127,14 +127,15 @@ class _ConvBlock(_EpochOnApply):
             raise NotImplementedError("native conv blocks are 3x3x3 only")
         bn = self.bn
         batch_stats = bn is not None and (self.training or not bn.track_running_stats)
-        params = (self.conv.weight,) + ((bn.weight, bn.bias) if bn is not None else ())
+        params = (self.conv.weight,) + ((bn.weight, bn.bias) if bn is not None else (self.conv.bias,))
         if batch_stats or ag.wants_grad(vol.data, None if skip is None else skip.data, *params):
             if vol.dtype == torch.float16:
                 raise NotImplementedError("precision 'fp16' is the inference pipeline; train in 'bf16' or 'fp32'")
             if out_dtype is not None and out_dtype != vol.dtype:
                 raise NotImplementedError("training path keeps one volume dtype")
             out = ag.ConvBlockFn.apply(vol.data, None if skip is None else skip.data, self.conv.weight,
-                                       None if bn is None else bn.weight, None if bn is None else bn.bias, self)
+                                       None if bn is None else bn.weight, None if bn is None else bn.bias,
+                                       self.conv.bias if bn is None else None, self)
             return G8Volume(out)
         impl = ops.conv_impl_for(self.in_channels, self.out_channels, self.stride, self.transposed)
         packed, scale, shift = self.prepared(impl, vol.dtype)
@@ -147,8 +148,8 @@ class _ConvBlock(_EpochOnApply):
             raise NotImplementedError(
                 "stand-alone Conv3d/Deconv3d forward is native for kernel 3, padding 1, channels % 8 == 0 only; "
                 "the 1x1x1 view-weight convs are fused into the warp/aggregate kernel (see DepthNet)")
-        vol = G8Volume.from_ncdhw(x, ops.volume_dtype())
-        return self.forward_g8(vol).to_ncdhw()
+        vol = G8Volume(ag.NcdhwToG8Fn.apply(x, ops.volume_dtype()))
+        return ag.G8ToNcdhwFn.apply(self.forward_g8(vol).data)
 
 
 class Conv3d(_ConvBlock):
@@ -265,7 +266,7 @@ class CostRegNet(_EpochOnApply):
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         """Reference call signature: [B,C,D,H,W] -> [B,1,D,H,W]."""
-        vol = G8Volume.from_ncdhw(x, ops.volume_dtype())
+        vol = G8Volume(ag.NcdhwToG8Fn.apply(x, ops.volume_dtype()))
         return self.forward_g8(vol).unsqueeze(1)
 
 
@@ -349,7 +350,11 @@ class AggWeightNetVolume(_EpochOnApply):
 def homo_warping(src_fea: torch.Tensor, src_proj: torch.Tensor, ref_proj: torch.Tensor,
                  depth_values: torch.Tensor) -> torch.Tensor:
     """Reference signature (models/module.py:297-302): src_fea [B,C,H,W], src_proj/ref_proj [B,4,4],
-    depth_values [B,D] or [B,D,H,W] -> warped volume [B,C,D,H,W]."""
+    depth_values [B,D] or [B,D,H,W] -> warped volume [B,C,D,H,W].  Forward only: the library has no stand-alone warp
+    backward (DepthNet differentiates the fused warp + aggregation instead), so inputs that require grad are rejected
+    rather than silently detached."""
+    if ag.wants_grad(src_fea, src_proj, ref_proj, depth_values):
+        raise NotImplementedError("homo_warping has no backward kernel; DepthNet's fused warp + aggregation is differentiable")
     rot_trans = ops.relative_rot_trans(src_proj.float(), ref_proj.float())
     return ops.homo_warp(ops.features_to_nhwc(src_fea), rot_trans, depth_values)
 
@@ -358,7 +363,7 @@ def depth_regression(p: torch.Tensor, depth_values: torch.Tensor) -> torch.Tenso
     """Reference signature (models/module.py:609-615): sum_d p * depth_values."""
     if depth_values.dim() == 1:
         depth_values = depth_values.view(1, -1).expand(p.shape[0], -1)
-    return ops.depth_regression(p, depth_values.to(torch.float32))
+    return ag.DepthRegressionFn.apply(p, depth_values.to(torch.float32))
 
 
 def uncertainty_aware_samples(cur_depth: torch.Tensor, exp_var: torch.Tensor, ndepth, dtype=None, device=None, shape=None) -> torch.Tensor:
