@@ -39,6 +39,10 @@ _SIGNATURES = {
     "damvs_warp_agg_fwd_f16": (c_int, [c_void_p, POINTER(c_void_p), c_int, c_void_p, c_void_p, c_void_p, c_void_p,
                                        c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "damvs_warp_gwc_fwd": (c_int, [c_void_p, POINTER(c_void_p), c_int, c_void_p, c_void_p, c_void_p] + [c_int] * 9 + [c_void_p]),
+    "damvs_warp_gwc_train_fwd": (c_int, [c_void_p, POINTER(c_void_p), c_int, c_void_p, c_void_p, c_void_p] + [c_int] * 8
+                                 + [c_void_p]),
+    "damvs_warp_gwc_bwd": (c_int, [c_void_p, POINTER(c_void_p), c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
+                                   POINTER(c_void_p)] + [c_int] * 7 + [c_void_p]),
     "damvs_conv3d_packed_weight_bytes": (c_size_t, [POINTER(ConvDesc)]),
     "damvs_conv3d_pack_weight": (c_int, [POINTER(ConvDesc), c_void_p, c_void_p, c_void_p]),
     "damvs_conv3d_fwd": (c_int, [POINTER(ConvDesc), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,

@@ -14,6 +14,8 @@ kernel of libdamvs_b200.so.
 * ``WarpAggFn``    fused warp + aggregation with a per-voxel weight net (eval-mode BN) or variance aggregation.
 * ``WarpAdaptiveTrainFn``  the adaptive aggregation when the weight net's BatchNorms use batch statistics: score ->
   native scalar chain -> weighted, one scatter pass in the backward (csrc/warp_agg_train.cu, csrc/wnet_chain.cu).
+* ``WarpGwcFn``    fused warp + group-wise correlation (not in the reference); forward and backward sample at the same
+  coordinates (csrc/warp_gwc_train.cu).
 """
 from __future__ import annotations
 
@@ -232,6 +234,24 @@ class WarpAggFn(torch.autograd.Function):
         wnet, rot_trans, dv, ref, *srcs = ctx.saved_tensors
         g_ref, g_srcs, g_wnet = ops_train.warp_agg_bwd(ref, srcs, rot_trans, dv, wnet, g_vol, ctx.mode)
         return (g_wnet, None, None, None, None, g_ref, *g_srcs)
+
+
+class WarpGwcFn(torch.autograd.Function):
+    """Fused warp + group-wise correlation -> G8 volume of max(groups, 8) channels.  Saves only its inputs; the
+    backward re-projects and re-samples (one scatter pass to the source features)."""
+
+    @staticmethod
+    def forward(ctx, rot_trans, depth_values, groups, out_dtype, ref, *srcs):
+        vol = ops_train.warp_gwc_train_fwd(ref, list(srcs), rot_trans, depth_values, groups, out_dtype)
+        ctx.groups = groups
+        ctx.save_for_backward(rot_trans, depth_values, ref, *srcs)
+        return vol
+
+    @staticmethod
+    def backward(ctx, g_vol):
+        rot_trans, dv, ref, *srcs = ctx.saved_tensors
+        g_ref, g_srcs = ops_train.warp_gwc_bwd(ref, srcs, rot_trans, dv, g_vol, ctx.groups)
+        return (None, None, None, None, g_ref, *g_srcs)
 
 
 class WarpAdaptiveTrainFn(torch.autograd.Function):

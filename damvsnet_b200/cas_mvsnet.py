@@ -6,7 +6,7 @@ fused warp+aggregate -> CostRegNet conv blocks -> softmax/regression head.
 """
 from __future__ import annotations
 
-from typing import Dict, List, Optional
+from typing import Dict, List, Optional, Sequence
 
 import torch
 import torch.nn as nn
@@ -15,19 +15,35 @@ from . import autograd as ag
 from . import ops
 from .module import AggWeightNetVolume, CostRegNet
 
-__all__ = ["DepthNet"]
+__all__ = ["DepthNet", "stage_volume_channels"]
+
+
+def stage_volume_channels(mode: str, in_channels: Sequence[int], groups: Optional[Sequence[int]]) -> List[int]:
+    """Channels of each stage's cost volume, i.e. CostRegNet's in_channels: the feature width, or for mode
+    "groupwise" max(G_s, 8) (a G = 4 volume is zero-padded to one 8-channel group).  `groups` holds one count per
+    stage, or fewer, the last repeated (as DepthNet reads it)."""
+    if mode != "groupwise":
+        return list(in_channels)
+    if groups is None:
+        raise ValueError('mode "groupwise" needs groups=(G per stage)')
+    gs = [int(g) for g in (groups if isinstance(groups, (list, tuple)) else [groups])]
+    return [max(gs[min(s, len(gs) - 1)], 8) for s in range(len(in_channels))]
 
 
 class DepthNet(nn.Module):
     """Per-stage cost-volume pipeline (reference models/cas_mvsnet.py:10-134)."""
 
-    def __init__(self, mode="adaptive", in_channels=None, groups=None):
+    def __init__(self, mode="adaptive", in_channels=None, groups=None, trainable: bool = False):
         """mode "variance" / "adaptive" are the reference's (models/cas_mvsnet.py:11-16).  mode "groupwise" with
         `groups` = per-stage group counts is NOT in the reference: the group-wise correlation cost volume BASELINE.json's
-        north star names (inference only; CostRegNet(in_channels=max(groups, 8)) consumes it)."""
+        north star names (CostRegNet(in_channels=max(groups, 8)) consumes it).  It is inference-only unless
+        `trainable` is set: then features that require grad go through the training kernels (csrc/warp_gwc_train.cu),
+        in fp32 or bf16; without grad the inference kernel runs either way.  `trainable` means nothing for the
+        other modes, which always train."""
         super().__init__()
         self.mode = mode
         assert mode in ("variance", "adaptive", "groupwise"), "Don't support {}!".format(mode)
+        self.trainable = bool(trainable)
         self.groups = None
         if mode == "groupwise":
             if groups is None:
@@ -51,11 +67,20 @@ class DepthNet(nn.Module):
         rot_trans = self.stage_rot_trans(proj_matrices)
         out_dtype = out_dtype or ops.volume_dtype()
         if self.mode == "groupwise":
+            g = self.groups[min(stage_idx, len(self.groups) - 1)]
             if ag.wants_grad(*features):
-                raise NotImplementedError("group-wise correlation is an inference-only variant (no backward kernel)")
+                if not self.trainable:
+                    raise NotImplementedError("group-wise correlation is an inference-only variant here: build "
+                                              "DepthNet(..., trainable=True) to train through it")
+                if out_dtype == torch.float16:
+                    raise NotImplementedError("precision 'fp16' is the inference pipeline; train in 'bf16' or 'fp32'")
+                with torch.no_grad():
+                    rot_trans = rot_trans.detach()      # the sampling grid is not differentiated (module.py:307)
+                    dv = depth_values.detach().contiguous()
+                nhwc = [ag.NhwcFn.apply(f) for f in features]
+                return ops.G8Volume(ag.WarpGwcFn.apply(rot_trans, dv, g, out_dtype, *nhwc))
             half = out_dtype in ops.HALF_DTYPES and ops.half_features()
             nhwc = ops.features_to_nhwc_half_multi(features) if half else [ops.features_to_nhwc(f) for f in features]
-            g = self.groups[min(stage_idx, len(self.groups) - 1)]
             return ops.warp_groupwise(nhwc[0], nhwc[1:], rot_trans, depth_values, g, out_dtype)
         wn = self.weight_net[stage_idx] if self.mode == "adaptive" else None
         batch_stats = wn is not None and wn.training

@@ -1,7 +1,7 @@
 """Tensor-level wrappers over the training-path entry points of the C ABI (include/damvs.h):
 BatchNorm statistics / apply / backward, convolution weight gradients, head backward, and the forward /
-backward kernels of the fused warp + aggregation.  Same conventions as ``ops.py``: CUDA tensors in, outputs
-allocated with torch, torch's current stream, no fallback.
+backward kernels of the fused warp + aggregation and of the fused warp + group-wise correlation.  Same conventions
+as ``ops.py``: CUDA tensors in, outputs allocated with torch, torch's current stream, no fallback.
 """
 from __future__ import annotations
 
@@ -174,6 +174,41 @@ def warp_agg_bwd(ref, srcs, rot_trans, depth_values, wnet, g_vol: torch.Tensor, 
                                                   _p(wnet), _p(g_vol.contiguous()), _dt(g_vol.dtype), _p(g_ref), _ptrs(g_srcs),
                                                   _p(g_wnet), b, c, d, h, w, m, per_pixel, _stream()))
     return g_ref, g_srcs, g_wnet
+
+
+def _gwc_common(ref, srcs, rot_trans, depth_values, groups: int):
+    b, h, w, c, d, dv, per_pixel = _warp_common(ref, srcs, rot_trans, depth_values)
+    if c not in (8, 16, 32) or groups not in (4, 8, 16, 32) or groups > c:
+        raise ValueError(f"group-wise correlation needs C in (8,16,32), groups in (4,8,16,32) and groups <= C; got C={c}, groups={groups}")
+    return b, h, w, c, d, dv, per_pixel
+
+
+def warp_gwc_train_fwd(ref, srcs, rot_trans, depth_values, groups: int, out_dtype: torch.dtype) -> torch.Tensor:
+    """Group-wise correlation at the training kernels' sampling coordinates -> G8 data tensor of max(groups, 8)
+    channels (fp32 or bf16; for groups = 4 channels 4..7 are zero)."""
+    b, h, w, c, d, dv, per_pixel = _gwc_common(ref, srcs, rot_trans, depth_values, groups)
+    if out_dtype not in _VOL_DTYPES:
+        raise ValueError("out_dtype must be fp32 or bf16")
+    out = torch.empty((b, max(groups, 8) // 8, d, h, w, 8), dtype=out_dtype, device=ref.device)
+    with torch.cuda.device_of(ref):
+        _lib.check(_lib.load().damvs_warp_gwc_train_fwd(_p(ref.contiguous()), _ptrs(srcs), len(srcs), _p(rot_trans.contiguous()), _p(dv),
+                                                        _p(out), b, c, groups, d, h, w, per_pixel, _dt(out_dtype), _stream()))
+    return out
+
+
+def warp_gwc_bwd(ref, srcs, rot_trans, depth_values, g_vol: torch.Tensor, groups: int):
+    """Backward of warp_gwc_train_fwd: (g_ref, [g_src]).  The padding channels of a groups = 4 g_vol are ignored."""
+    b, h, w, c, d, dv, per_pixel = _gwc_common(ref, srcs, rot_trans, depth_values, groups)
+    g_vol = g_vol.contiguous()
+    if _vol_dims(g_vol) != (b, max(groups, 8), d, h, w):
+        raise ValueError(f"g_vol must be a G8 volume [B,{max(groups, 8) // 8},D,H,W,8]")
+    g_ref = torch.empty_like(ref)
+    g_srcs = [torch.zeros_like(s) for s in srcs]
+    with torch.cuda.device_of(ref):
+        _lib.check(_lib.load().damvs_warp_gwc_bwd(_p(ref.contiguous()), _ptrs(srcs), len(srcs), _p(rot_trans.contiguous()), _p(dv),
+                                                  _p(g_vol), _dt(g_vol.dtype), _p(g_ref), _ptrs(g_srcs), b, c, groups, d, h, w,
+                                                  per_pixel, _stream()))
+    return g_ref, g_srcs
 
 
 def warp_score_fwd(ref, srcs, rot_trans, depth_values, w1: torch.Tensor) -> torch.Tensor:

@@ -20,7 +20,7 @@ from typing import Dict, List, Sequence, Tuple
 import torch
 
 from . import synthetic
-from .cas_mvsnet import DepthNet
+from .cas_mvsnet import DepthNet, stage_volume_channels
 from .module import CostRegNet
 
 StageInput = Tuple[List[torch.Tensor], torch.Tensor, torch.Tensor]
@@ -29,15 +29,18 @@ StageInput = Tuple[List[torch.Tensor], torch.Tensor, torch.Tensor]
 class HotPathRunner:
     def __init__(self, state_dict: Dict[str, torch.Tensor], mode: str = "adaptive",
                  in_channels: Sequence[int] = synthetic.STAGE_CHANNELS, base_channels: Sequence[int] = (8, 8, 8),
-                 device: torch.device | str = "cuda:0"):
+                 device: torch.device | str = "cuda:0", groups: Sequence[int] | None = None):
+        """mode "groupwise" (not in the reference) takes `groups` = per-stage group counts; the state dict then holds
+        CostRegNets of in_channels max(G, 8), as HotPathTrainer(mode="groupwise") trains them."""
         self.device = torch.device(device)
         self.mode = mode
-        self.depthnet = DepthNet(mode, list(in_channels)).eval()
+        vol_channels = stage_volume_channels(mode, in_channels, groups)
+        self.depthnet = DepthNet(mode, list(in_channels), groups).eval()
         if mode == "adaptive":
             self.depthnet.load_state_dict({k[len("DepthNet."):]: v for k, v in state_dict.items()
                                            if k.startswith("DepthNet.")}, strict=True)
         self.cost_regularization = torch.nn.ModuleList(
-            [CostRegNet(c, b) for c, b in zip(in_channels, base_channels)]).eval()
+            [CostRegNet(c, b) for c, b in zip(vol_channels, base_channels)]).eval()
         self.cost_regularization.load_state_dict({k[len("cost_regularization."):]: v for k, v in state_dict.items()
                                                   if k.startswith("cost_regularization.")}, strict=True)
         self.depthnet.to(self.device)

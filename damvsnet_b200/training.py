@@ -25,7 +25,7 @@ import torch.distributed as dist
 import torch.nn.functional as F
 
 from . import synthetic
-from .cas_mvsnet import DepthNet
+from .cas_mvsnet import DepthNet, stage_volume_channels
 from .module import CostRegNet
 
 StageInput = Tuple[List[torch.Tensor], torch.Tensor, torch.Tensor]
@@ -161,15 +161,19 @@ def depth_loss(outputs: Sequence[Dict[str, torch.Tensor]], depth_gt: Sequence[to
 
 
 class HotPathTrainer:
-    """DepthNet + per-stage CostRegNets in train() mode, Adam (train.py:439), one bucketed gradient all-reduce."""
+    """DepthNet + per-stage CostRegNets in train() mode, Adam (train.py:439), one bucketed gradient all-reduce.
+    mode "groupwise" (not in the reference) takes `groups` = per-stage group counts; its cost volume has no parameters,
+    so only the CostRegNets (in_channels = max(G, 8)) train."""
 
     def __init__(self, state_dict: Optional[Dict[str, torch.Tensor]] = None, mode: str = "adaptive",
                  in_channels: Sequence[int] = synthetic.STAGE_CHANNELS, base_channels: Sequence[int] = (8, 8, 8),
-                 device: torch.device | str = "cuda:0", lr: float = 1e-3, weight_decay: float = 0.0, group=None):
+                 device: torch.device | str = "cuda:0", lr: float = 1e-3, weight_decay: float = 0.0, group=None,
+                 groups: Optional[Sequence[int]] = None):
         self.device = torch.device(device)
         self.group = group
-        self.depthnet = DepthNet(mode, list(in_channels))
-        self.cost_regularization = torch.nn.ModuleList([CostRegNet(c, b) for c, b in zip(in_channels, base_channels)])
+        vol_channels = stage_volume_channels(mode, in_channels, groups)
+        self.depthnet = DepthNet(mode, list(in_channels), groups, trainable=True)
+        self.cost_regularization = torch.nn.ModuleList([CostRegNet(c, b) for c, b in zip(vol_channels, base_channels)])
         if state_dict is not None:
             if mode == "adaptive":
                 self.depthnet.load_state_dict({k[len("DepthNet."):]: v for k, v in state_dict.items()

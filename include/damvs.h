@@ -142,6 +142,23 @@ int damvs_warp_gwc_fwd(const void* ref_nhwc, const void* const* src_nhwc, int n_
                        const float* depth_hyp, void* out_vol, int B, int C, int G, int D, int H, int W,
                        int per_pixel_hyp, int feat_dtype, int out_dtype, void* stream);
 
+/* ---- group-wise correlation, training forward and backward ---------------------------------------------------
+ * The forward and the backward sample at bit-identical coordinates (the reference's operation order, as the other
+ * training kernels), so the gradient is that of the volume the forward returned.  S = C/G, k = 1/(n_src S):
+ *   fwd: out_vol[g] = k sum_v sum_{c in g} ref[c] warp_v[c]; fp32 NHWC features, G8 volume of max(G, 8) channels in
+ *        out_dtype = DAMVS_F32 | DAMVS_BF16 (G = 4: channels 4..7 written as zero).
+ *   bwd: g_vol (G8, g_dtype = DAMVS_F32 | DAMVS_BF16; padding channels of G = 4 are ignored) ->
+ *        g_ref[c] = k sum_d g_vol[g(c)] sum_v warp_v[c]  (overwritten),
+ *        g_src[v] += bilinear scatter of k g_vol[g(c)] ref[c]  (ACCUMULATED with vector atomics: zero them first;
+ *        HOST array of device pointers).  The sampling grid and the hypotheses receive no gradient.
+ * C in {8,16,32}, G in {4,8,16,32}, G <= C, n_src in [1,15].  Other arguments as damvs_warp_agg_fwd.             */
+int damvs_warp_gwc_train_fwd(const float* ref_nhwc, const float* const* src_nhwc, int n_src, const float* rot_trans,
+                             const float* depth_hyp, void* out_vol, int B, int C, int G, int D, int H, int W,
+                             int per_pixel_hyp, int out_dtype, void* stream);
+int damvs_warp_gwc_bwd(const float* ref_nhwc, const float* const* src_nhwc, int n_src, const float* rot_trans,
+                       const float* depth_hyp, const void* g_vol, int g_dtype, float* g_ref, float* const* g_src, int B,
+                       int C, int G, int D, int H, int W, int per_pixel_hyp, void* stream);
+
 /* ---- fused `prob` convolution + head ------------------------------------------
  * CostRegNet's last layer (models/module.py:530: Conv3d 8 -> 1, k3, p1, no bias) and the softmax / regression /
  * confidence / variance head (models/cas_mvsnet.py:105-124) in ONE launch: the logits stay in shared memory.

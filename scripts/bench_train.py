@@ -3,7 +3,7 @@
 per GPU, D=48/32/8, forward + backward through warp / cost volume / CostRegNet / head with batch-statistics
 BatchNorm, bucketed NCCL gradient all-reduce, Adam step.  Not the headline metric (bench.py is); one JSON line.
 
-    python scripts/bench_train.py [--steps K] [--warmup W] [--batch 4]
+    python scripts/bench_train.py [--steps K] [--warmup W] [--batch 4] [--mode adaptive|variance|groupwise --groups 8,8,4]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         scripts/bench_train.py --gpus N
 """
@@ -32,6 +32,9 @@ def main():
     ap.add_argument("--ndepths", default="48,32,8")
     ap.add_argument("--precision", default="bf16", choices=["bf16", "fp32"])
     ap.add_argument("--detail", action="store_true")
+    ap.add_argument("--mode", default="adaptive", choices=["adaptive", "variance", "groupwise"],
+                    help="cost-volume aggregation; groupwise (not in the reference) needs --groups")
+    ap.add_argument("--groups", default=None, help="group-wise correlation groups per stage, e.g. 8,8,4")
     args = ap.parse_args()
 
     import torch.distributed as dist
@@ -46,10 +49,19 @@ def main():
     import damvsnet_b200 as dm
     from damvsnet_b200 import _lib, synthetic
     from damvsnet_b200.runner import make_workload
+    from damvsnet_b200.cas_mvsnet import stage_volume_channels
     from damvsnet_b200.training import HotPathTrainer
     dm.set_precision(args.precision)
     nd = [int(x) for x in args.ndepths.split(",")]
-    trainer = HotPathTrainer(synthetic.hot_path_state_dict(seed=0), device=dev)
+    groups = [int(x) for x in args.groups.split(",")] if args.groups else None
+    if args.mode == "groupwise":
+        if groups is None:
+            ap.error("--mode groupwise needs --groups")
+        vol_channels = stage_volume_channels(args.mode, synthetic.STAGE_CHANNELS, groups)
+        sd = synthetic.hot_path_state_dict(in_channels=vol_channels, seed=0, mode=args.mode)
+    else:
+        sd = synthetic.hot_path_state_dict(seed=0, mode=args.mode)
+    trainer = HotPathTrainer(sd, mode=args.mode, device=dev, groups=groups)
     stages = make_workload(args.height, args.width, args.nviews, nd, batch=args.batch, seed=rank, device=dev)
     # features come out of the (PyTorch) FPN in real training and need gradients: keep that work in the step
     stages = [([f.requires_grad_(True) for f in fs], p, d) for fs, p, d in stages]
@@ -108,7 +120,10 @@ def main():
             depth_loss(trainer.forward(stages), gts, masks).backward()
         detail = {"forward_ms": timed(fwd), "forward_backward_ms": timed(fwd_bwd)}
     if rank == 0:
-        print(json.dumps({"metric": "training samples/sec, hot path fwd+bwd+allreduce+Adam at 512x640 N=5 D=48/32/8", "value": world * args.batch / (ms_step / 1e3),
+        metric = "training samples/sec, hot path fwd+bwd+allreduce+Adam at 512x640 N=5 D=48/32/8"
+        if args.mode != "adaptive":     # the default keeps its metric name (and output) unchanged
+            metric += f", {args.mode} aggregation" + (f" groups {args.groups}" if args.mode == "groupwise" else "")
+        print(json.dumps({"metric": metric, "value": world * args.batch / (ms_step / 1e3),
                           "unit": "samples/s", "n_gpus": world, "steps": args.steps, "ms_per_step": ms_step, "scaling": "weak",
                           "dtype": args.precision, "data": "synthetic", "loss": float(loss), "gpu_launches": int(launches),
                           "config": {"workload": f"DTU-train {args.height}x{args.width}, N={args.nviews}, D={args.ndepths}, batch {args.batch}/GPU (BASELINE.json configs[3])",
