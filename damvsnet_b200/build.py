@@ -27,11 +27,6 @@ NVCC_FLAGS = [
 ]
 
 
-# development aid: DAMVS_TC_TRACE_BUILD=1 compiles the per-CTA timestamp probes into conv3d_tc.cu (see DAMVS_TC_TRACE)
-if os.environ.get("DAMVS_TC_TRACE_BUILD"):
-    NVCC_FLAGS.append("-DDAMVS_TC_TRACE_BUILD")
-
-
 def sources():
     return sorted(os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith(".cu"))
 

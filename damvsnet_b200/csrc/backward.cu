@@ -10,7 +10,6 @@
 // The data gradient of a conv block is one more forward-type convolution (transposed roles), run by the
 // existing conv kernels with re-packed weights -- see damvsnet_b200/autograd.py.
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -160,8 +159,7 @@ extern "C" int damvs_conv3d_wgrad(const damvs_conv3d_desc* d, const void* x, con
   DAMVS_CUDA_OK(cudaMemsetAsync(dw, 0, (size_t)d->Cin * d->Cout * 27 * sizeof(float), st));
   {
     // bf16 volumes: tensor-core kernel (wgrad_mma.cu); everything else: the fp32 CUDA-core kernel below
-    static const bool no_mma = getenv("DAMVS_WGRAD_NO_MMA") != nullptr;   // development knob
-    const int rc = no_mma ? DAMVS_ERR_UNSUPPORTED : conv_wgrad_mma_launch(d, x, g_y, dw, st);
+    const int rc = conv_wgrad_mma_launch(d, x, g_y, dw, st);
     if (rc != DAMVS_ERR_UNSUPPORTED) return rc;
   }
   const bool xf = d->in_dtype == DAMVS_F32, gf = d->out_dtype == DAMVS_F32;

@@ -50,13 +50,6 @@ inline int current_sm_count() {
   return n;
 }
 
-// Development knob DAMVS_TC_GRID_PCT: cap the persistent conv grids at pct % of (CTAs per SM x SMs), so that some SMs
-// keep room for other streams' kernels (experiment of DESIGN.md section 6; 100 = off).
-inline int tc_grid_cap(int ctas) {
-  static const int pct = getenv("DAMVS_TC_GRID_PCT") ? atoi(getenv("DAMVS_TC_GRID_PCT")) : 100;
-  return pct >= 100 ? ctas : (ctas * pct + 99) / 100;
-}
-
 // ---- G8 volume addressing ---------------------------------------------------
 // element offset of channel 0 of group g at voxel (z,y,x) of batch item b
 __host__ __device__ inline size_t g8_offset(int b, int g, int z, int y, int x, int G, int D, int H, int W) {

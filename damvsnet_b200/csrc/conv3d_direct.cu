@@ -12,7 +12,6 @@
 // the 27*Cin*8 weights of that group sit in shared memory and are read as
 // warp-wide broadcasts; input voxels are 8-channel vectors of the G8 volume.
 #include <algorithm>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -213,11 +212,10 @@ int conv3d_direct_launch(const damvs_conv3d_desc* d, const void* in, const void*
     P.Dout = (d->Din - 1) / d->stride + 1; P.Hout = (d->Hin - 1) / d->stride + 1; P.Wout = (d->Win - 1) / d->stride + 1;
   }
   const int Gout = (d->Cout + 7) / 8;
-  // voxels per thread: as many as a row has 32-voxel strips to give (coarse levels are 50..100 wide)
-  // measured on B200 (fp32 pipeline at the DTU-test shape): 34.1 / 43.0 / 41.7 views/s for 1 / 2 / 4 voxels per thread
-  // (4 costs occupancy: 128 registers), hence 2 wherever a row has two 32-voxel strips
-  static const int vx_cap = getenv("DAMVS_DIRECT_VX") ? atoi(getenv("DAMVS_DIRECT_VX")) : 2;   // development knob
-  const int vx = std::min(vx_cap, P.Wout >= 96 ? 4 : (P.Wout >= 48 ? 2 : 1));
+  // voxels per thread (coarse levels are 50..100 wide); measured on B200 (fp32 pipeline at the DTU-test shape): 34.1 /
+  // 43.0 / 41.7 views/s for 1 / 2 / 4 voxels per thread (4 costs occupancy: 128 registers), hence 2 wherever a row has
+  // two 32-voxel strips
+  const int vx = P.Wout >= 48 ? 2 : 1;
   const long long ctas = (long long)P.Dout * ((P.Hout + 3) / 4) * ((P.Wout + 32 * vx - 1) / (32 * vx));
   if (ctas > 0x7fffffffll) return set_error(DAMVS_ERR_UNSUPPORTED, "conv3d direct: volume too large for one launch");
   dim3 grid((unsigned)ctas, Gout, d->B);
@@ -232,7 +230,7 @@ int conv3d_direct_launch(const damvs_conv3d_desc* d, const void* in, const void*
   } while (0)
 #define LAUNCH(TI, TO)                                                                                          \
   do {                                                                                                          \
-    if (vx == 4) LAUNCH_V(TI, TO, 4); else if (vx == 2) LAUNCH_V(TI, TO, 2); else LAUNCH_V(TI, TO, 1);          \
+    if (vx == 2) LAUNCH_V(TI, TO, 2); else LAUNCH_V(TI, TO, 1);                                                 \
   } while (0)
   const bool out_f32 = d->plain_out || d->out_dtype == DAMVS_F32;
   const bool one = d->plain_out && smem <= 48 * 1024;   // Cout == 1 (checked by the C ABI); Cin <= 48 keeps the default smem limit

@@ -34,7 +34,6 @@
 // epilogue (TMEM -> registers -> kw combine -> BN affine / ReLU / skip -> 16-byte stores).
 // Accumulators are double buffered in TMEM so the epilogue of plane z overlaps the MMAs of plane z+1.
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 #include <vector>
 
@@ -81,8 +80,6 @@ struct TcParams {
   int n0, Cout, relu, plain_out, niter, nsteps, nslots;
   int tiles_x, tiles_y, ntiles;  // persistent CTAs walk tiles blockIdx.x, blockIdx.x + gridDim.x, ...
   int zchunks, zlen;             // a tile covers zlen iterations (depth planes) of one of zchunks depth ranges
-  unsigned long long* trace;  // development aid: per-CTA event timestamps (null in production)
-  int dbg;                    // development aid (DAMVS_TC_DBG, trace builds only): bit0 skip epilogue body, bit1 skip MMA issue, bit2 skip loads
 };
 
 __host__ __device__ inline int steps_offset() { return (int)sizeof(PackedHeader); }
@@ -98,24 +95,6 @@ struct Geo {
   __host__ __device__ static constexpr int rows0(int MC) { return MODE == MODE_S1 ? 4 * MC + 2 : (MODE == MODE_T ? 4 * MC + 1 : 4 * MC); }
   __host__ __device__ static constexpr int rows1(int MC) { return MODE == MODE_S2 ? 4 * MC + 1 : 0; }
 };
-
-__device__ __forceinline__ unsigned long long gtime() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-  return t;
-}
-// Per-CTA event timestamps for DAMVS_TC_TRACE (development aid): compiled in only with -DDAMVS_TC_TRACE_BUILD, so the
-// production epilogue carries no timer reads, predicates or stores.
-#ifdef DAMVS_TC_TRACE_BUILD
-#define TRACE(slot_)                                                                                              \
-  do {                                                                                                            \
-    if (P.trace) P.trace[((size_t)blockIdx.x) * 64 + (slot_)] = gtime();                \
-  } while (0)
-#define DBG(bit_) (P.dbg & (bit_))
-#else
-#define TRACE(slot_) do { } while (0)
-#define DBG(bit_) false
-#endif
 
 __device__ __forceinline__ float shfl_dn(uint32_t v, int d) { return __uint_as_float(__shfl_down_sync(0xffffffffu, v, d)); }
 
@@ -251,7 +230,6 @@ __global__ void __launch_bounds__(320) conv3d_tc_kernel(const __grid_constant__ 
   const int ty0 = ((t2_ / P.tiles_x) % P.tiles_y) * TH;                  \
   const int tx0 = (t2_ % P.tiles_x) * G_::TW;
 
-  if (threadIdx.x == 0) { TRACE(0); }
   // ---- one-time setup ------------------------------------------------------------------------
   // The weights (up to 110 KB for the 64-channel layers) arrive by bulk copies issued below, off the critical path: the
   // per-CTA timelines of the coarse layers showed 4.5-7 us of a 10-15 us CTA life spent in a ld.global / st.shared loop.
@@ -285,7 +263,6 @@ __global__ void __launch_bounds__(320) conv3d_tc_kernel(const __grid_constant__ 
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   const int niter = P.niter;
-  if (threadIdx.x == 0) { TRACE(1); }
 
   if (warp == 0) {
     // ===== TMA producer =====
@@ -297,11 +274,6 @@ __global__ void __launch_bounds__(320) conv3d_tc_kernel(const __grid_constant__ 
       const int nplanes = (nit - 1) * G_::adv + G_::span;
       for (int k = 0; k < nplanes; ++k) {
         if (round > 0) mbar_wait(&empty[slot], (round - 1) & 1);
-        if (DBG(4)) {   // development aid: no loads, the MMAs run on whatever the ring holds
-          mbar_arrive_expect_tx(&full[slot], 0);
-          if (++slot == nslots) { slot = 0; ++round; }
-          continue;
-        }
         mbar_arrive_expect_tx(&full[slot], bytes);
         uint8_t* dst = sA + slot * slot_stride;
         const int plane = it0 * G_::adv + k + G_::p0;
@@ -336,18 +308,16 @@ __global__ void __launch_bounds__(320) conv3d_tc_kernel(const __grid_constant__ 
         ++next_wait;
         if (++wait_slot == nslots) { wait_slot = 0; ++wait_round; }
       }
-      if (leader && acc_n < 12) { TRACE(4 + acc_n); }
       const int buf = NBUF == 2 ? (acc_n & 1) : 0;
       if (acc_n >= NBUF) mbar_wait(&tmem_empty[buf], (NBUF == 2 ? ((acc_n >> 1) - 1) : (acc_n - 1)) & 1);
       tc_fence_after();
-      if (leader && acc_n < 12) { TRACE(16 + acc_n); }
       const uint32_t dbase = tmem_base + buf * ACC_COLS;
       int s1 = base_slot + 1; if (s1 >= nslots) s1 -= nslots;
       int s2 = base_slot + 2; if (s2 >= nslots) s2 -= nslots;
       const uint32_t so0 = a_base16 + base_slot * slot16;
       const uint32_t so1 = a_base16 + s1 * slot16;
       const uint32_t so2 = a_base16 + s2 * slot16;
-      issue_iteration<MODE, CP, MC, G, F16>(leader && !DBG(2), so0, so1, so2, b_base16, dbase);
+      issue_iteration<MODE, CP, MC, G, F16>(leader, so0, so1, so2, b_base16, dbase);
       if (leader) {
         mma_commit(&tmem_full[buf]);
 #pragma unroll
@@ -441,11 +411,10 @@ __global__ void __launch_bounds__(320) conv3d_tc_kernel(const __grid_constant__ 
         }
         mbar_wait(&tmem_full[buf], (NBUF == 2 ? (acc_n >> 1) : acc_n) & 1);
         tc_fence_after();
-        if (warp == 2 && lane == 0 && acc_n < 12) { TRACE(28 + acc_n); }
 #pragma unroll
         for (int u = 0; u < U; ++u) {
           const int k = u / (MC * CPG), c = (u / CPG) % MC, ng = u % CPG;
-          if (ng >= ngroups || DBG(1)) continue;   // uniform
+          if (ng >= ngroups) continue;   // uniform
           const int pdh = 2 * half + k;
           const uint32_t cbase = tbase + (pdh * MC + c) * N + ng * 8;
           uint32_t ya[8], yb[8], yc[8];  // tw = 1 (even x), tw = 2 (odd x, same input), tw = 0 (odd x, input + 1)
@@ -485,12 +454,11 @@ __global__ void __launch_bounds__(320) conv3d_tc_kernel(const __grid_constant__ 
         }
         mbar_wait(&tmem_full[buf], (NBUF == 2 ? (acc_n >> 1) : acc_n) & 1);
         tc_fence_after();
-        if (warp == 2 && lane == 0 && acc_n < 12) { TRACE(28 + acc_n); }
 #pragma unroll
         for (int u = 0; u < U; ++u) {
           const int c = MC >= 2 ? half * (MC / 2) + u / CPG : 0;
           const int ng = MC >= 2 ? u % CPG : 2 * u + half;
-          if (ng >= ngroups || DBG(1)) continue;   // uniform
+          if (ng >= ngroups) continue;   // uniform
           const uint32_t cbase = tbase + c * N + ng * 8;
           if (P.plain_out) {
             uint32_t y0, y1, y2;
@@ -525,7 +493,6 @@ __global__ void __launch_bounds__(320) conv3d_tc_kernel(const __grid_constant__ 
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty[buf]);
-      if (warp == 2 && lane == 0 && acc_n < 12) { TRACE(40 + acc_n); }
     }
     }
   }
@@ -537,7 +504,6 @@ __global__ void __launch_bounds__(320) conv3d_tc_kernel(const __grid_constant__ 
     tc_fence_after();
     tmem_dealloc(tmem_base, TMEM_COLS);
   }
-  if (threadIdx.x == 32) TRACE(2);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -722,11 +688,6 @@ static EncodeTiledFn encode_fn() {
   return fn;
 }
 
-static CUtensorMapL2promotion l2_promotion() {
-  static const int v = getenv("DAMVS_TC_L2") ? atoi(getenv("DAMVS_TC_L2")) : 2;   // development knob
-  return v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : v == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-}
-
 // G8 bf16 volume [BG][D][H][W*8] viewed with rows (row0, row0 + row_step, ...)
 static int make_map(CUtensorMap* m, const void* base, int BG, int D, int H, int W, int row0, int row_step, int box_rows, int G, bool f16) {
   EncodeTiledFn fn = encode_fn();
@@ -738,7 +699,7 @@ static int make_map(CUtensorMap* m, const void* base, int BG, int D, int H, int 
   cuuint32_t estr[4] = {1, 1, 1, 1};
   void* addr = (void*)((const uint8_t*)base + (size_t)row0 * W * 16);
   CUresult r = fn(m, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, addr, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  CU_TENSOR_MAP_SWIZZLE_NONE, l2_promotion(), CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                  CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return set_error(DAMVS_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) W=%d H=%d D=%d BG=%d rows=%d", (int)r, W, H, D, BG, box_rows);
   return DAMVS_OK;
 }
@@ -751,6 +712,10 @@ static size_t fixed_smem(int CP, int nsteps) {
   return (size_t)nsteps * 2 * 3 * CP * 16 + 2 * CP * sizeof(float) + (2 * kMaxSlots + 5) * sizeof(uint64_t) + 16;
 }
 constexpr size_t kSmemBudget = 227 * 1024;
+// at most 8 planes in the ring (the TMA runs up to 8 - span planes ahead): a deeper ring only takes shared memory from
+// co-resident CTAs
+constexpr int kSlotCap = 8;
+static_assert(kSlotCap <= kMaxSlots, "barrier arrays hold kMaxSlots slots");
 
 template <int MODE, int CP, int MC, int G, bool F16>
 static int launch_one(const damvs_conv3d_desc* d, TcParams& P, const void* in, const std::vector<StepSrc>& steps, cudaStream_t st) {
@@ -768,13 +733,7 @@ static int launch_one(const damvs_conv3d_desc* d, TcParams& P, const void* in, c
   }
   // ring depth: TMA runs ahead of the MMAs by nslots - span planes
   const size_t sb = slot_bytes(MODE, G, MC), fx = fixed_smem(CP, nsteps);
-  int nslots = (int)((kSmemBudget - fx) / sb);
-  const int nplanes = (P.niter - 1) * G_::adv + G_::span;
-  if (nslots > kMaxSlots) nslots = kMaxSlots;
-  static const int slot_cap = getenv("DAMVS_TC_SLOTS") ? atoi(getenv("DAMVS_TC_SLOTS")) : 8;   // development knob
-  static const int l2promo = getenv("DAMVS_TC_L2") ? atoi(getenv("DAMVS_TC_L2")) : 2;
-  (void)l2promo;
-  if (nslots > slot_cap) nslots = std::max(slot_cap, G_::span + 1);
+  int nslots = std::min((int)((kSmemBudget - fx) / sb), kSlotCap);
   if (nslots < G_::span + 1) return set_error(DAMVS_ERR_UNSUPPORTED, "conv3d tcgen05: ring does not fit");
   // leave room for a second CTA per SM when a deep ring is not needed
   while (nslots > G_::span + 1 && fx + (size_t)nslots * sb + 1024 > kSmemBudget / 2) --nslots;
@@ -791,9 +750,8 @@ static int launch_one(const damvs_conv3d_desc* d, TcParams& P, const void* in, c
   // flight (3.54 -> 3.48 ms) and costs throughput with 3-4 views in flight (more CTAs contending), hence the low bar.
   {
     const int spatial = P.tiles_x * P.tiles_y * d->B;
-    static const int zsplit_off = getenv("DAMVS_TC_NO_ZSPLIT") != nullptr;   // development knob
     int zc = 1;
-    if (!zsplit_off && spatial * 2 < 148) {
+    if (spatial * 2 < 148) {
       const int want = (148 + spatial - 1) / spatial;
       const int min_len = spatial * 4 < 148 ? 1 : 2;
       zc = std::max(1, std::min(want, P.niter / min_len));
@@ -812,43 +770,7 @@ static int launch_one(const damvs_conv3d_desc* d, TcParams& P, const void* in, c
   constexpr int NEEDC = nbuf_of(MODE, CP, ACC) * ACC;
   constexpr int TCOLS = NEEDC <= 32 ? 32 : NEEDC <= 64 ? 64 : NEEDC <= 128 ? 128 : NEEDC <= 256 ? 256 : 512;
   occ = std::max(1, std::min(occ, 512 / TCOLS));
-  static const int occ_cap = getenv("DAMVS_TC_OCC") ? atoi(getenv("DAMVS_TC_OCC")) : 8;   // development knob
-  occ = std::min(occ, occ_cap);
-  const int num_sms = current_sm_count();
-  dim3 grid((unsigned)std::min(P.ntiles, tc_grid_cap(occ * num_sms)), 1, 1);
-#ifdef DAMVS_TC_TRACE_BUILD
-  // Development aid, compiled ONLY into a -DDAMVS_TC_TRACE_BUILD library: timestamps of a few CTAs, printed to stderr.
-  // It allocates and synchronises, which the product C ABI never does (and which would break graph capture).
-  const char* tr = getenv("DAMVS_TC_TRACE");
-  if (tr) {
-    const size_t n = (size_t)grid.x * 64;
-    unsigned long long* dbuf = nullptr;
-    DAMVS_CUDA_OK(cudaMalloc(&dbuf, n * 8));
-    DAMVS_CUDA_OK(cudaMemsetAsync(dbuf, 0, n * 8, st));
-    P.trace = dbuf;
-    kern<<<grid, 320, smem, st>>>(m0, m1, P);
-    DAMVS_LAUNCH_OK("conv3d_tc kernel (trace)");
-    DAMVS_CUDA_OK(cudaStreamSynchronize(st));
-    std::vector<unsigned long long> h(n);
-    DAMVS_CUDA_OK(cudaMemcpy(h.data(), dbuf, n * 8, cudaMemcpyDeviceToHost));
-    DAMVS_CUDA_OK(cudaFree(dbuf));
-    P.trace = nullptr;
-    unsigned long long t0 = ~0ull, t1 = 0;
-    for (size_t c = 0; c < n / 64; ++c) { if (h[c * 64]) t0 = std::min(t0, h[c * 64]); t1 = std::max(t1, h[c * 64 + 2]); }
-    fprintf(stderr, "[tc trace] mode %d CP %d MC %d G %d grid %u tiles %d niter %d nslots %d smem %zu: kernel span %.1f us\n", MODE, CP, MC, G, grid.x,
-            P.ntiles, P.niter, nslots, smem, (t1 - t0) / 1e3);
-    const size_t picks[3] = {0, n / 64 / 2, n / 64 - 1};
-    for (size_t pi = 0; pi < 3; ++pi) {
-      const unsigned long long* e = &h[picks[pi] * 64];
-      fprintf(stderr, "  cta %zu: start +%.1f us, setup %.2f, life %.2f us | iter: ", picks[pi], (e[0] - t0) / 1e3, (e[1] - e[0]) / 1e3, (e[2] - e[0]) / 1e3);
-      for (int it = 0; it < P.niter && it < 12; ++it)
-        fprintf(stderr, "[%d mma_rdy %.2f acc_free %.2f epi_start %.2f epi_end %.2f] ", it, (e[4 + it] - e[0]) / 1e3, (e[16 + it] - e[0]) / 1e3,
-                (e[28 + it] - e[0]) / 1e3, (e[40 + it] - e[0]) / 1e3);
-      fprintf(stderr, "\n");
-    }
-    return DAMVS_OK;
-  }
-#endif
+  dim3 grid((unsigned)std::min(P.ntiles, occ * current_sm_count()), 1, 1);
   kern<<<grid, 320, smem, st>>>(m0, m1, P);
   DAMVS_LAUNCH_OK("conv3d_tc kernel");
   return DAMVS_OK;
@@ -907,11 +829,7 @@ int conv3d_tc_launch(const damvs_conv3d_desc* d, const void* in, const void* pac
   if (!build_program(mode, G, steps)) return set_error(DAMVS_ERR_UNSUPPORTED, "conv3d tcgen05: no program for Cin=%d", d->Cin);
   const int nsteps = (int)steps.size();
   const size_t bb = (blob_bytes(nsteps, CP) + 255) / 256 * 256;
-  int mc = pick_mc(mode, G, CP, nsteps, mode == MODE_T ? d->Hin : P.Hout, mode == MODE_T ? d->Win : P.Wout, d->B);
-  static const int mc_force = getenv("DAMVS_TC_MC") ? atoi(getenv("DAMVS_TC_MC")) : 0;   // development knobs
-  static const int dbg = getenv("DAMVS_TC_DBG") ? atoi(getenv("DAMVS_TC_DBG")) : 0;
-  if (mc_force && mc_force < mc && mc_fits(mode, G, CP, nsteps, mc_force)) mc = mc_force;
-  P.dbg = dbg;
+  const int mc = pick_mc(mode, G, CP, nsteps, mode == MODE_T ? d->Hin : P.Hout, mode == MODE_T ? d->Win : P.Wout, d->B);
   if (mc == 0) return set_error(DAMVS_ERR_UNSUPPORTED, "conv3d tcgen05: Cin=%d Cout=%d does not fit in shared memory", d->Cin, d->Cout);
   for (int k = 0; k < split; ++k) {
     P.blob = (const uint8_t*)packed + k * bb;
@@ -920,10 +838,8 @@ int conv3d_tc_launch(const damvs_conv3d_desc* d, const void* in, const void* pac
 #define GO(MODE_, CP_, MC_, G_)                                   \
   if (mode == MODE_ && CP == CP_ && mc == MC_ && G == G_)         \
     rc = f16 ? launch_one<MODE_, CP_, MC_, G_, true>(d, P, in, steps, st) : launch_one<MODE_, CP_, MC_, G_, false>(d, P, in, steps, st)
-    // the layer shapes of CostRegNet with base_channels 8 (reference models/module.py:513-530)
-    GO(MODE_S1, 16, 2, 1); GO(MODE_S1, 16, 1, 1);   // conv0 (stage 3), prob
-    GO(MODE_S1, 16, 2, 2); GO(MODE_S1, 16, 1, 2);   // conv0 (stage 2), conv2
-    GO(MODE_S1, 16, 2, 4); GO(MODE_S1, 16, 1, 4);   // conv0 (stage 1)
+    // the layer shapes of CostRegNet with base_channels 8 (reference models/module.py:513-530); stride-1 layers with
+    // Cout <= 16 (conv0, conv2, prob) run on conv3d_tcf.cu / conv3d_tcp.cu
     GO(MODE_S1, 32, 1, 4);                           // conv4
     GO(MODE_S1, 32, 1, 1);                           // adjoint of conv0 (stage 1): 8 -> 32
     GO(MODE_S1, 32, 1, 8);                           // conv6 (two output halves)

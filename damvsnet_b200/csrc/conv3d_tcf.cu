@@ -3,7 +3,7 @@
 // Same operation and data layout as conv3d_tc.cu (out = skip + relu(conv(in) * scale + shift), G8 bf16 volumes,
 // TMA plane loads, kw folded into N and recombined by two shuffles in the epilogue) for the layers with at most 16
 // output channels (CostRegNet conv0, conv2, prob and the adjoint convolutions of that shape, reference
-// models/module.py:513-530).  Measured on those layers (DAMVS_TC_DBG experiments, DESIGN.md section 3.2): the MMA
+// models/module.py:513-530).  Measured on those layers (phase knock-out experiments, DESIGN.md section 3.2): the MMA
 // phase alone takes as long as the whole kernel, at ~66 cycles per M128 x N48 x K16 instruction of which ~32 are
 // the 4 KB A-operand read from shared memory -- every input plane is read 9 times, once per (kd, kh) tap.
 // Here an iteration is one INPUT plane: its three (kh) tap reads feed all three depth taps at once,
@@ -19,7 +19,6 @@
 // Barriers: full[slot] (TMA -> MMA), done[slot] (ONE tcgen05.commit per iteration: it frees the plane's slot for the
 // producer and tells the epilogue that output plane p - 1 is complete) and acc_empty[ring slot] (epilogue -> MMA).
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 #include <vector>
 
@@ -353,9 +352,8 @@ static int launch_g(const damvs_conv3d_desc* d, Params& P, const void* in, cudaS
   if (r != CUDA_SUCCESS) return set_error(DAMVS_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
   const size_t sb = (size_t)G * R0 * kP * 16, fx = fixed_smem(G, S_::N3);
   // ring of 8 planes when two CTAs per SM still fit, else 4 (a power of two: the epilogue maps an iteration to its slot)
-  static const int cap = getenv("DAMVS_TCF_SLOTS") ? atoi(getenv("DAMVS_TCF_SLOTS")) : 8;   // development knob: 4 or 8
   const size_t room = ((227 * 1024) / 2 - fx - 1024) / sb;
-  P.log_nslots = (room >= 8 && cap >= 8) ? 3 : 2;
+  P.log_nslots = room >= 8 ? 3 : 2;
   const int nslots = 1 << P.log_nslots;
   const size_t smem = fx + (size_t)nslots * sb;
   auto kern = conv3d_tcf_kernel<G, CPN, F16>;
@@ -364,9 +362,7 @@ static int launch_g(const damvs_conv3d_desc* d, Params& P, const void* in, cudaS
   P.tiles_x = (d->Win + TW - 1) / TW;
   P.tiles_y = (d->Hin + TH - 1) / TH;
   P.ntiles = P.tiles_x * P.tiles_y * d->B;
-  const int num_sms = current_sm_count();
-  static const int occ_cap = getenv("DAMVS_TC_OCC") ? atoi(getenv("DAMVS_TC_OCC")) : 2;   // development knob
-  dim3 grid((unsigned)std::min(P.ntiles, tc_grid_cap(std::min(2, occ_cap) * num_sms)), 1, 1);
+  dim3 grid((unsigned)std::min(P.ntiles, 2 * current_sm_count()), 1, 1);   // two CTAs per SM (256 TMEM columns each)
   kern<<<grid, 320, smem, st>>>(m0, P);
   DAMVS_LAUNCH_OK("conv3d_tcf kernel");
   return DAMVS_OK;
@@ -376,8 +372,7 @@ static int launch_g(const damvs_conv3d_desc* d, Params& P, const void* in, cudaS
 
 // ---- entry points used by conv3d_tc.cu's dispatch ------------------------------------------------------------------
 bool conv3d_tcf_supported(const damvs_conv3d_desc* d) {
-  static const bool off = getenv("DAMVS_TC_NO_FOLD") != nullptr;   // development knob
-  if (off || d->transposed || d->stride != 1 || d->Cout > 16 || d->Cin % 8) return false;
+  if (d->transposed || d->stride != 1 || d->Cout > 16 || d->Cin % 8) return false;
   const int G = d->Cin / 8;
   return G == 1 || G == 2 || G == 4;
 }

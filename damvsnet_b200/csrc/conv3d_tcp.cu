@@ -17,12 +17,11 @@
 // Warp roles (320 threads): warp 0 TMA producer, warp 1 MMA issuer (one thread), warps 2-9 epilogue in two groups of
 // four; group g drains the output planes with global index = g mod 2, so the two planes an iteration completes are
 // drained concurrently (four groups / 16 epilogue warps measured slower: their barrier spinning takes issue slots from
-// the issuer).  Measured (DAMVS_TCP_DBG phase elimination, DESIGN.md section 3.2): the issuer's instruction
+// the issuer).  Measured (phase knock-out experiments, DESIGN.md section 3.2): the issuer's instruction
 // path per iteration is what bounds these kernels once the A reads are gone, hence one wait for the planes, one for
 // the accumulator pair, at most four MMAs and ONE commit per iteration (the same barrier frees the shared-memory slot
 // for the producer and publishes the completed output planes to the epilogue).
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 
 #include "common.cuh"
@@ -57,7 +56,7 @@ struct Params {
   const uint8_t* blob;
   float* out;
   int B, D, H, W;
-  int tiles_x, tiles_y, ntiles, dbg;
+  int tiles_x, tiles_y, ntiles;
   uint32_t fmt_xor;   // 0 for bf16 operands; the A / B format bits of the instruction descriptor for fp16 (XOR turns them off)
   // fused head (HEAD = true): per-pixel hypotheses in, probability volume and the three maps out; `out` is unused
   const float* hyp;
@@ -166,16 +165,14 @@ __global__ void __launch_bounds__(THREADS, 2) conv3d_tcp_kernel(const __grid_con
           const uint32_t blo = b_base16 | ((uint32_t)B_ROWS << 16);                                     // LBO = 64 rows * 16 B
           const uint32_t d_old = tmem_base + ((m - 1) & (RING / 2 - 1)) * (2 * NBP), d_new = tmem_base + (m & (RING / 2 - 1)) * (2 * NBP);
           const bool first = i == 0, last = i == NIT - 1;
-          if (!(P.dbg & 1)) {
 #pragma unroll
-            for (int c = 0; c < MC; ++c) {
-              const uint64_t adesc = ((uint64_t)DESC_HI << 32) | (alo + c * 128);
-              // a tile's first pair only touches plane 0 (block 1), and starts it
-              mma_bf16_ss(d_old + c * (RING * NBP) + (first ? NBP : 0), adesc, ((uint64_t)DESC_HI << 32) | (blo + (first ? NBP : 0)),
-                          idesc_bf16_m128(first ? NBP : 2 * NBP) ^ P.fmt_xor, first ? 0u : 1u);
-              // its last pair only touches plane D - 1 (block 2)
-              mma_bf16_ss(d_new + c * (RING * NBP), adesc, ((uint64_t)DESC_HI << 32) | (blo + 2 * NBP), idesc_bf16_m128(last ? NBP : 2 * NBP) ^ P.fmt_xor, 0u);
-            }
+          for (int c = 0; c < MC; ++c) {
+            const uint64_t adesc = ((uint64_t)DESC_HI << 32) | (alo + c * 128);
+            // a tile's first pair only touches plane 0 (block 1), and starts it
+            mma_bf16_ss(d_old + c * (RING * NBP) + (first ? NBP : 0), adesc, ((uint64_t)DESC_HI << 32) | (blo + (first ? NBP : 0)),
+                        idesc_bf16_m128(first ? NBP : 2 * NBP) ^ P.fmt_xor, first ? 0u : 1u);
+            // its last pair only touches plane D - 1 (block 2)
+            mma_bf16_ss(d_new + c * (RING * NBP), adesc, ((uint64_t)DESC_HI << 32) | (blo + 2 * NBP), idesc_bf16_m128(last ? NBP : 2 * NBP) ^ P.fmt_xor, 0u);
           }
           mma_commit(&done[slot]);   // the plane pair can be overwritten; output planes 2i - 1, 2i (and D - 1 at the end) are complete
         }
@@ -221,7 +218,6 @@ __global__ void __launch_bounds__(THREADS, 2) conv3d_tcp_kernel(const __grid_con
         mbar_wait(&done[g & (NS - 1)], (g >> LOG_NS) & 1u);
         tc_fence_after();
         const uint32_t pair = ((gz + 1) >> 1) & (RING / 2 - 1);
-        if (P.dbg & 2) { tc_fence_before(); if (lane == 0) mbar_arrive(&acc_empty[pair]); continue; }
         uint32_t y[MC][8], y8[MC];   // taps kh * 3 + kw = 0..7 and 8
 #pragma unroll
         for (int c = 0; c < MC; ++c) {
@@ -357,8 +353,7 @@ constexpr int kHeadMaxD = 64;   // D * 1 KB of logits per CTA: two CTAs per SM u
 
 // ---- entry points used by conv3d_tc.cu's dispatch ------------------------------------------------------------------
 bool conv3d_tcp_supported(const damvs_conv3d_desc* d) {
-  static const bool off = getenv("DAMVS_TC_NO_FOLD") != nullptr || getenv("DAMVS_TC_NO_PROB") != nullptr;   // development knobs
-  return !off && d->plain_out && !d->transposed && d->stride == 1 && d->Cin == 8;   // the layer; odd depths are launched on conv3d_tcf.cu
+  return d->plain_out && !d->transposed && d->stride == 1 && d->Cin == 8;   // the layer; odd depths are launched on conv3d_tcf.cu
 }
 
 size_t conv3d_tcp_packed_bytes(const damvs_conv3d_desc*) { return (sizeof(tcp::Header) + 2 * tcp::B_ROWS * 16 + 255) / 256 * 256; }
@@ -393,14 +388,10 @@ static int tcp_launch_impl(const damvs_conv3d_desc* d, const void* in, const voi
   auto kern = conv3d_tcp_kernel<HEAD>;
   DAMVS_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   DAMVS_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  static const int dbg = getenv("DAMVS_TCP_DBG") ? atoi(getenv("DAMVS_TCP_DBG")) : 0;   // development knob: 1 = no MMAs, 2 = no epilogue work
-  P.dbg = dbg;
   P.tiles_x = (d->Win + TW - 1) / TW;
   P.tiles_y = (d->Hin + TH - 1) / TH;
   P.ntiles = P.tiles_x * P.tiles_y * d->B;
-  const int num_sms = current_sm_count();
-  static const int occ_cap = getenv("DAMVS_TC_OCC") ? atoi(getenv("DAMVS_TC_OCC")) : 2;   // development knob
-  dim3 grid((unsigned)std::min(P.ntiles, tc_grid_cap(std::min(2, occ_cap) * num_sms)), 1, 1);
+  dim3 grid((unsigned)std::min(P.ntiles, 2 * current_sm_count()), 1, 1);   // two CTAs per SM (__launch_bounds__)
   kern<<<grid, THREADS, smem, st>>>(m0, P);
   DAMVS_LAUNCH_OK(HEAD ? "conv3d_tcp kernel (fused head)" : "conv3d_tcp kernel");
   return DAMVS_OK;

@@ -9,7 +9,6 @@
 // k is a coalesced 128-byte line per warp.  A pixel's column is strided by H*W
 // in memory; the main kernel stages a D x 128-pixel tile in shared memory with
 // cp.async, a streaming kernel covers any D / alignment.
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -228,8 +227,7 @@ extern "C" int damvs_softmax_regress_fwd(const float* logits, const float* depth
   cudaStream_t st = (cudaStream_t)stream;
   unsigned blocks = (unsigned)((total + 255) / 256);
   const bool aligned = (HW % 4 == 0) && aligned16(logits) && aligned16(depth_hyp) && B <= 65535;
-  static const bool no_reg = getenv("DAMVS_HEAD_STAGED") != nullptr;   // development knob: A/B against the staged kernel
-  if (!no_reg && per_pixel_hyp && B <= 65535 && (D == 8 || D == 16 || D == 32 || D == 48 || D == 64 || D == 96)) {
+  if (per_pixel_hyp && B <= 65535 && (D == 8 || D == 16 || D == 32 || D == 48 || D == 64 || D == 96)) {
     // small maps (stage 1: 115 k pixels) get 64-thread CTAs: twice the CTAs to spread over the 148 SMs
     const int threads = total < 148ll * 8 * 128 ? 64 : 128;
     dim3 grid((unsigned)((HW + threads - 1) / threads), B);

@@ -154,7 +154,7 @@ __device__ __forceinline__ Tap8 load_tap8(const float* p) {
 //     block most of the time (sub-pixel steps along the epipolar line): the taps stay in registers and are
 //     only re-fetched when the block changes;
 //   * the per-channel math runs on packed fp32x2 instructions.
-template <int C, int MODE, typename OutT, int DCH, bool PF>
+template <int C, int MODE, typename OutT, int DCH>
 __global__ void __launch_bounds__(128) warp_agg_kernel(const WarpAggParams P) {
   constexpr int LPP = C / 8;     // lanes per pixel
   constexpr int PPW = 32 / LPP;  // pixels per warp (along x)
@@ -271,18 +271,6 @@ __global__ void __launch_bounds__(128) warp_agg_kernel(const WarpAggParams P) {
             t11 = load_tap8(p + (long long)W * C + C);
             cur = off;
           }
-          if (PF && j + 1 < DCH) {  // pull the next hypothesis' tap lines towards L1 while this one is blended
-            const int offn = LPP > 1 ? s_fo[warp][pw][j + 1] : fp[j + 1 < DCH ? j + 1 : j].off;
-            if (offn != off) {
-              const float* pn = img + offn;
-              asm volatile("prefetch.global.L1 [%0];" ::"l"(pn));
-              asm volatile("prefetch.global.L1 [%0];" ::"l"(pn + (long long)W * C));
-              if (C * 4 * 2 > 128 || (((size_t)pn & 127) + C * 8 > 128)) {
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(pn + C));
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(pn + (long long)W * C + C));
-              }
-            }
-          }
           const float2 a00 = splat(fwt.x), a01 = splat(fwt.y), a10 = splat(fwt.z), a11 = splat(fwt.w);
           float2 wv[4];
 #pragma unroll
@@ -372,11 +360,11 @@ static int launch_warp_agg(const WarpAggParams& P, int out_dtype, cudaStream_t s
   constexpr int TW = 32 / (C / 8), TH = 4, DCH = 4;
   dim3 grid((P.W + TW - 1) / TW, (P.H + TH - 1) / TH, P.B);
   if (out_dtype == DAMVS_F32)
-    warp_agg_kernel<C, MODE, float, DCH, false><<<grid, 128, 0, st>>>(P);
+    warp_agg_kernel<C, MODE, float, DCH><<<grid, 128, 0, st>>>(P);
   else if (out_dtype == DAMVS_F16)
-    warp_agg_kernel<C, MODE, __half, DCH, false><<<grid, 128, 0, st>>>(P);
+    warp_agg_kernel<C, MODE, __half, DCH><<<grid, 128, 0, st>>>(P);
   else
-    warp_agg_kernel<C, MODE, __nv_bfloat16, DCH, false><<<grid, 128, 0, st>>>(P);
+    warp_agg_kernel<C, MODE, __nv_bfloat16, DCH><<<grid, 128, 0, st>>>(P);
   DAMVS_LAUNCH_OK("warp_agg kernel");
   return DAMVS_OK;
 }

@@ -14,14 +14,12 @@
 //     into the projection rows once per CTA;
 //   * footprints (packed fp16 weights + byte offset, 16 bytes) are exchanged between the lanes of a pixel through
 //     shared memory in a [depth][pixel] layout, one conflict-free LDS.128 per use.
-// Kept from the fp32 kernel: thread = (pixel, 8 channels), depth chunks with (view, depth) loop order and tap reuse
-// while consecutive hypotheses stay inside one 2x2 block, packed fp32x2 math after the blend, 16-byte stores.
+// Kept from the fp32 kernel: thread = (pixel, 8 channels), depth chunks with (view, depth) loop order, packed fp32x2
+// math after the blend, 16-byte stores.  Unlike the fp32 kernel, every hypothesis loads its taps (see HCfg).
 //
 // Sampling semantics are unchanged (zero padding per tap, no z > 0 mask, NaN coordinates sample zero); coordinates
 // differ from the reference's by fp32 rounding only (<= 1e-4 pixel at W = 1600).
 #include <cuda_fp16.h>
-
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -105,21 +103,16 @@ __device__ __forceinline__ void store1(__half* p, float v) { *reinterpret_cast<u
 
 __device__ __forceinline__ uint4 ldg16(const void* p) { return __ldg(reinterpret_cast<const uint4*>(p)); }
 
-// CPT = channels per thread (8 or 16): with 16 a thread owns two G8 groups -- the per-(view, hypothesis) overheads
-// (footprint exchange, tap addressing, the weight-net chain, loop control) are amortised over twice the channels, which
-// is what an instruction-issue-bound kernel needs (stage 2: 220 -> ~155 instructions per (view, voxel, 16 channels)).
-template <int C, int CPT, int MODE, typename OutT, int DCH, bool REUSE, int MINB, bool FULL, int G = 0>
+template <int C, int MODE, typename OutT, int DCH, int MINB, bool FULL, int G = 0>
 __global__ void __launch_bounds__(128, MINB) warp_agg_h_kernel(const WarpAggHParams P) {
-  // group-wise correlation (MODE == kAggGwc, CPT == 8): G groups of GS channels; a thread's 8 channels cover NV groups,
+  // group-wise correlation (MODE == kAggGwc): G groups of GS channels; a thread's 8 channels cover NV groups,
   // or an eighth / quarter / half of one group that LPG adjacent lanes finish with shuffles
   constexpr int GS = G > 0 ? C / G : 8;
   constexpr int NV = GS >= 8 ? 1 : 8 / GS;
   constexpr int LPG = GS >= 8 ? GS / 8 : 1;
   constexpr int GOUT = G > 0 && G < 8 ? 8 : (G > 0 ? G : 8);
-  static_assert(MODE != kAggGwc || (CPT == 8 && G > 0), "group-wise correlation runs with 8 channels per thread");
-  constexpr int NG = CPT / 8;      // G8 groups per thread
-  constexpr int HP = CPT / 2;      // channel pairs per thread
-  constexpr int LPP = C / CPT;     // lanes per pixel
+  static_assert(MODE != kAggGwc || G > 0, "group-wise correlation needs a group count");
+  constexpr int LPP = C / 8;       // lanes per pixel
   constexpr int PPW = 32 / LPP;    // pixels per warp (along x)
   constexpr int TW = PPW, TH = 4;
   constexpr int NPJ = (DCH + LPP - 1) / LPP;
@@ -151,33 +144,32 @@ __global__ void __launch_bounds__(128, MINB) warp_agg_h_kernel(const WarpAggHPar
   const size_t img_bytes = (size_t)HW * C * 2;
 
   // -ref in fp32: the blend chain starts from it, so the chain ends in (warp - ref)
-  float nrf[CPT];
-#pragma unroll
-  for (int n = 0; n < NG; ++n) {
-    const uint4 r = ldg16(reinterpret_cast<const char*>(P.ref) + (size_t)b * img_bytes + ((size_t)y * W + x) * (C * 2) + q * (CPT * 2) + n * 16);
+  float nrf[8];
+  {
+    const uint4 r = ldg16(reinterpret_cast<const char*>(P.ref) + (size_t)b * img_bytes + ((size_t)y * W + x) * (C * 2) + q * 16);
     const __half2* h = reinterpret_cast<const __half2*>(&r);
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
       const float2 f = __half22float2(h[k]);
-      nrf[n * 8 + 2 * k] = -f.x; nrf[n * 8 + 2 * k + 1] = -f.y;
+      nrf[2 * k] = -f.x; nrf[2 * k + 1] = -f.y;
     }
   }
   const float fx = (float)x, fy = (float)y;
-  float2 w1[HP];
+  float2 w1[4];
   float s1 = 0.f, b1 = 0.f, w2 = 0.f, s2 = 0.f, b2 = 0.f;
   if (MODE == DAMVS_AGG_ADAPTIVE) {
 #pragma unroll
-    for (int j = 0; j < HP; ++j) w1[j] = make_float2(s_wnet[q * CPT + 2 * j], s_wnet[q * CPT + 2 * j + 1]);
+    for (int j = 0; j < 4; ++j) w1[j] = make_float2(s_wnet[q * 8 + 2 * j], s_wnet[q * 8 + 2 * j + 1]);
     s1 = s_wnet[C]; b1 = s_wnet[C + 1]; w2 = s_wnet[C + 2]; s2 = s_wnet[C + 3]; b2 = s_wnet[C + 4];
   }
   const float* hyp = P.per_pixel ? P.hyp + (long long)b * D * HW + (long long)y * W + x : P.hyp + (long long)b * D;
   const long long hyp_stride = P.per_pixel ? HW : 1;
-  OutT* out = reinterpret_cast<OutT*>(P.out) + g8_offset(b, q * NG, 0, y, x, C / 8, D, H, W);
-  const long long out_stride = HW * 8, grp_stride = (long long)D * HW * 8;
+  OutT* out = reinterpret_cast<OutT*>(P.out) + g8_offset(b, q, 0, y, x, C / 8, D, H, W);
+  const long long out_stride = HW * 8;
   const float inv_n = 1.f / (float)(n_src + 1), inv_nsrc = 1.f / (float)n_src;
 
   for (int d0 = 0; d0 < D; d0 += DCH) {
-    float2 acc[DCH][HP], sq[MODE == DAMVS_AGG_VARIANCE ? DCH : 1][HP];
+    float2 acc[DCH][4], sq[MODE == DAMVS_AGG_VARIANCE ? DCH : 1][4];
     float accg[MODE == kAggGwc ? DCH : 1][NV];
     if (MODE == kAggGwc) {
 #pragma unroll
@@ -188,7 +180,7 @@ __global__ void __launch_bounds__(128, MINB) warp_agg_h_kernel(const WarpAggHPar
 #pragma unroll
     for (int j = 0; j < DCH; ++j)
 #pragma unroll
-      for (int k = 0; k < HP; ++k) {
+      for (int k = 0; k < 4; ++k) {
         if (MODE == DAMVS_AGG_VARIANCE) {
           acc[j][k] = make_float2(-nrf[2 * k], -nrf[2 * k + 1]);
           sq[j][k] = make_float2(nrf[2 * k] * nrf[2 * k], nrf[2 * k + 1] * nrf[2 * k + 1]);
@@ -221,11 +213,7 @@ __global__ void __launch_bounds__(128, MINB) warp_agg_h_kernel(const WarpAggHPar
         }
       }
       if (LPP > 1) __syncwarp();
-      const char* img = reinterpret_cast<const char*>(P.src[v]) + (size_t)b * img_bytes + q * (CPT * 2);
-      int cur = -1;
-      uint4 t00[NG], t01[NG], t10[NG], t11[NG];
-#pragma unroll
-      for (int n = 0; n < NG; ++n) t00[n] = t01[n] = t10[n] = t11[n] = make_uint4(0, 0, 0, 0);
+      const char* img = reinterpret_cast<const char*>(P.src[v]) + (size_t)b * img_bytes + q * 16;
 #pragma unroll
       for (int j = 0; j < DCH; ++j) {
         if (FULL || d0 + j < D) {  // uniform
@@ -236,60 +224,49 @@ __global__ void __launch_bounds__(128, MINB) warp_agg_h_kernel(const WarpAggHPar
           } else {
             f = fp[j];
           }
-          if (!REUSE || f.off != cur) {
-            const char* p = img + f.off;
+          const char* p = img + f.off;
+          const uint4 t00 = ldg16(p), t01 = ldg16(p + C * 2);
+          const uint4 t10 = ldg16(p + (size_t)W * (C * 2)), t11 = ldg16(p + (size_t)W * (C * 2) + C * 2);
+          float df[8], base[8];   // warp - ref  (variance mode: warp)
 #pragma unroll
-            for (int n = 0; n < NG; ++n) {
-              t00[n] = ldg16(p + n * 16);
-              t01[n] = ldg16(p + C * 2 + n * 16);
-              t10[n] = ldg16(p + (size_t)W * (C * 2) + n * 16);
-              t11[n] = ldg16(p + (size_t)W * (C * 2) + C * 2 + n * 16);
-            }
-            cur = f.off;
-          }
-          float2 e[HP], sv = make_float2(0.f, 0.f);
+          for (int k = 0; k < 8; ++k) base[k] = MODE == DAMVS_AGG_ADAPTIVE ? nrf[k] : 0.f;
+          fhfma8<false>(df, base, t00, f.w01);
+          fhfma8<true>(df, df, t01, f.w01);
+          fhfma8<false>(df, df, t10, f.w23);
+          fhfma8<true>(df, df, t11, f.w23);
+          if (MODE == kAggGwc) {
+            float pr[8];                                   // ref * warp (nrf holds -ref)
 #pragma unroll
-          for (int n = 0; n < NG; ++n) {
-            float df[8], base[8];   // warp - ref  (variance mode: warp)
+            for (int k = 0; k < 8; ++k) pr[k] = -nrf[k] * df[k];
+            if (GS >= 8) {
+              float s = ((pr[0] + pr[1]) + (pr[2] + pr[3])) + ((pr[4] + pr[5]) + (pr[6] + pr[7]));
 #pragma unroll
-            for (int k = 0; k < 8; ++k) base[k] = MODE == DAMVS_AGG_ADAPTIVE ? nrf[n * 8 + k] : 0.f;
-            fhfma8<false>(df, base, t00[n], f.w01);
-            fhfma8<true>(df, df, t01[n], f.w01);
-            fhfma8<false>(df, df, t10[n], f.w23);
-            fhfma8<true>(df, df, t11[n], f.w23);
-            if (MODE == kAggGwc) {
-              float pr[8];                                   // ref * warp (nrf holds -ref)
+              for (int o = LPG / 2; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+              accg[j][0] += s;
+            } else {
 #pragma unroll
-              for (int k = 0; k < 8; ++k) pr[k] = -nrf[k] * df[k];
-              if (GS >= 8) {
-                float s = ((pr[0] + pr[1]) + (pr[2] + pr[3])) + ((pr[4] + pr[5]) + (pr[6] + pr[7]));
+              for (int k = 0; k < NV; ++k) {
+                float s = 0.f;
 #pragma unroll
-                for (int o = LPG / 2; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-                accg[j][0] += s;
-              } else {
-#pragma unroll
-                for (int k = 0; k < NV; ++k) {
-                  float s = 0.f;
-#pragma unroll
-                  for (int i = 0; i < GS; ++i) s += pr[k * GS + i];
-                  accg[j][k] += s;
-                }
+                for (int i = 0; i < GS; ++i) s += pr[k * GS + i];
+                accg[j][k] += s;
               }
-              continue;
             }
+          } else if (MODE == DAMVS_AGG_VARIANCE) {
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
               const float2 d2 = make_float2(df[2 * k], df[2 * k + 1]);
-              if (MODE == DAMVS_AGG_VARIANCE) {
-                acc[j][n * 4 + k] = __fadd2_rn(acc[j][n * 4 + k], d2);
-                sq[j][n * 4 + k] = __ffma2_rn(d2, d2, sq[j][n * 4 + k]);
-              } else {
-                e[n * 4 + k] = __fmul2_rn(d2, d2);                          // cas_mvsnet.py:66
-                sv = __ffma2_rn(w1[n * 4 + k], e[n * 4 + k], sv);          // 1x1x1 conv C->1
-              }
+              acc[j][k] = __fadd2_rn(acc[j][k], d2);
+              sq[j][k] = __ffma2_rn(d2, d2, sq[j][k]);
             }
-          }
-          if (MODE == DAMVS_AGG_ADAPTIVE) {
+          } else {
+            float2 e[4], sv = make_float2(0.f, 0.f);
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+              const float2 d2 = make_float2(df[2 * k], df[2 * k + 1]);
+              e[k] = __fmul2_rn(d2, d2);                          // cas_mvsnet.py:66
+              sv = __ffma2_rn(w1[k], e[k], sv);                   // 1x1x1 conv C->1
+            }
             float s = sv.x + sv.y;
 #pragma unroll
             for (int o = LPP / 2; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
@@ -297,7 +274,7 @@ __global__ void __launch_bounds__(128, MINB) warp_agg_h_kernel(const WarpAggHPar
             const float wtv = fmaxf(fmaf(a * w2, s2, b2), 0.f) + 1.f;         // conv 1->1, BN, ReLU; (weight + 1)
             const float2 wt = make_float2(wtv, wtv);
 #pragma unroll
-            for (int k = 0; k < HP; ++k) acc[j][k] = __ffma2_rn(wt, e[k], acc[j][k]);   // cas_mvsnet.py:73-76
+            for (int k = 0; k < 4; ++k) acc[j][k] = __ffma2_rn(wt, e[k], acc[j][k]);   // cas_mvsnet.py:73-76
           }
         }
       }
@@ -341,24 +318,21 @@ __global__ void __launch_bounds__(128, MINB) warp_agg_h_kernel(const WarpAggHPar
 #pragma unroll
     for (int j = 0; j < DCH; ++j) {
       if (FULL || d0 + j < D) {
+        F8 r;
 #pragma unroll
-        for (int n = 0; n < NG; ++n) {
-          F8 r;
-#pragma unroll
-          for (int k = 0; k < 4; ++k) {
-            float2 a;
-            const float2 ac = acc[j][n * 4 + k];
-            if (MODE == DAMVS_AGG_VARIANCE) {
-              const float2 m = make_float2(ac.x * inv_n, ac.y * inv_n);
-              const float2 qq = sq[j][n * 4 + k];
-              a = make_float2(fmaf(qq.x, inv_n, -m.x * m.x), fmaf(qq.y, inv_n, -m.y * m.y));   // cas_mvsnet.py:85
-            } else {
-              a = make_float2(ac.x * inv_nsrc, ac.y * inv_nsrc);                                // cas_mvsnet.py:87
-            }
-            r.v[2 * k] = a.x; r.v[2 * k + 1] = a.y;
+        for (int k = 0; k < 4; ++k) {
+          float2 a;
+          const float2 ac = acc[j][k];
+          if (MODE == DAMVS_AGG_VARIANCE) {
+            const float2 m = make_float2(ac.x * inv_n, ac.y * inv_n);
+            const float2 qq = sq[j][k];
+            a = make_float2(fmaf(qq.x, inv_n, -m.x * m.x), fmaf(qq.y, inv_n, -m.y * m.y));   // cas_mvsnet.py:85
+          } else {
+            a = make_float2(ac.x * inv_nsrc, ac.y * inv_nsrc);                                // cas_mvsnet.py:87
           }
-          if (live) store8(out + n * grp_stride + (long long)(d0 + j) * out_stride, r);
+          r.v[2 * k] = a.x; r.v[2 * k + 1] = a.y;
         }
+        if (live) store8(out + (long long)(d0 + j) * out_stride, r);
       }
     }
   }
@@ -419,34 +393,28 @@ __global__ void __launch_bounds__(128) nchw_to_nhwc_f16_kernel(const __grid_cons
   }
 }
 
-// Per channel width: channels per thread, depth chunk and minimum CTAs per SM (measured at the DTU-test stage shapes on
-// B200: unconditional tap loads let the compiler batch a chunk's gathers, which beats skipping repeated 2x2 blocks; the
-// narrow kernels trade accumulators for occupancy; 16 channels per thread saves ~30 % of the instructions but costs
-// more in occupancy at 128 registers -- 488 vs 403 us at stage 1, 528 vs 515 us at stage 2).
-template <int C> struct HCfg { static constexpr int CPT = 8, DCH = 4, MINB = 1; };
-template <> struct HCfg<32> { static constexpr int CPT = 8, DCH = 4, MINB = 5; };
-template <> struct HCfg<16> { static constexpr int CPT = 8, DCH = 2, MINB = 6; };
-template <> struct HCfg<8> { static constexpr int CPT = 8, DCH = 2, MINB = 8; };
-
-template <int C, int MODE, int CPT, int DCH, int MINB>
-static int launch_h_cfg(const WarpAggHParams& P, int out_dtype, cudaStream_t st) {
-  constexpr int TW = 32 / (C / CPT), TH = 4;
-  dim3 grid((P.W + TW - 1) / TW, (P.H + TH - 1) / TH, P.B);
-  const bool full = P.D % DCH == 0;
-  if (out_dtype == DAMVS_F32) warp_agg_h_kernel<C, CPT, MODE, float, DCH, false, 1, false><<<grid, 128, 0, st>>>(P);
-  else if (out_dtype == DAMVS_F16 && full) warp_agg_h_kernel<C, CPT, MODE, __half, DCH, false, MINB, true><<<grid, 128, 0, st>>>(P);
-  else if (out_dtype == DAMVS_F16) warp_agg_h_kernel<C, CPT, MODE, __half, DCH, false, MINB, false><<<grid, 128, 0, st>>>(P);
-  else if (full) warp_agg_h_kernel<C, CPT, MODE, __nv_bfloat16, DCH, false, MINB, true><<<grid, 128, 0, st>>>(P);
-  else warp_agg_h_kernel<C, CPT, MODE, __nv_bfloat16, DCH, false, MINB, false><<<grid, 128, 0, st>>>(P);
-  DAMVS_LAUNCH_OK("warp_agg_h kernel");
-  return DAMVS_OK;
-}
+// Per channel width: depth chunk and minimum CTAs per SM (measured at the DTU-test stage shapes on B200: unconditional
+// tap loads let the compiler batch a chunk's gathers, which beats skipping repeated 2x2 blocks; the narrow kernels trade
+// accumulators for occupancy).  Eight channels per thread: 16 (two G8 groups per thread) saves ~30 % of the instructions
+// but costs more in occupancy at 128 registers -- 488 vs 403 us at stage 1, 528 vs 515 us at stage 2.
+template <int C> struct HCfg { static constexpr int DCH = 4, MINB = 1; };
+template <> struct HCfg<32> { static constexpr int DCH = 4, MINB = 5; };
+template <> struct HCfg<16> { static constexpr int DCH = 2, MINB = 6; };
+template <> struct HCfg<8> { static constexpr int DCH = 2, MINB = 8; };
 
 template <int C, int MODE>
 static int launch_h(const WarpAggHParams& P, int out_dtype, cudaStream_t st) {
-  static const int cfg = getenv("DAMVS_WARP_CFG") ? atoi(getenv("DAMVS_WARP_CFG")) : 0;   // development knob
-  if (C >= 16 && cfg == 16) return launch_h_cfg<C, MODE, (C >= 16 ? 16 : 8), 2, 4>(P, out_dtype, st);   // 16 channels per thread
-  return launch_h_cfg<C, MODE, HCfg<C>::CPT, HCfg<C>::DCH, HCfg<C>::MINB>(P, out_dtype, st);
+  constexpr int DCH = HCfg<C>::DCH, MINB = HCfg<C>::MINB;
+  constexpr int TW = 32 / (C / 8), TH = 4;
+  dim3 grid((P.W + TW - 1) / TW, (P.H + TH - 1) / TH, P.B);
+  const bool full = P.D % DCH == 0;
+  if (out_dtype == DAMVS_F32) warp_agg_h_kernel<C, MODE, float, DCH, 1, false><<<grid, 128, 0, st>>>(P);
+  else if (out_dtype == DAMVS_F16 && full) warp_agg_h_kernel<C, MODE, __half, DCH, MINB, true><<<grid, 128, 0, st>>>(P);
+  else if (out_dtype == DAMVS_F16) warp_agg_h_kernel<C, MODE, __half, DCH, MINB, false><<<grid, 128, 0, st>>>(P);
+  else if (full) warp_agg_h_kernel<C, MODE, __nv_bfloat16, DCH, MINB, true><<<grid, 128, 0, st>>>(P);
+  else warp_agg_h_kernel<C, MODE, __nv_bfloat16, DCH, MINB, false><<<grid, 128, 0, st>>>(P);
+  DAMVS_LAUNCH_OK("warp_agg_h kernel");
+  return DAMVS_OK;
 }
 
 // Group-wise correlation on the tuned kernel (fp16 features, 2-byte volume, D a multiple of the depth chunk); called by
@@ -456,16 +424,15 @@ static int launch_gwc_fast_cg(const WarpAggHParams& P, int out_dtype, cudaStream
   constexpr int DCH = HCfg<C>::DCH, MINB = HCfg<C>::MINB;
   constexpr int TW = 32 / (C / 8), TH = 4;
   dim3 grid((P.W + TW - 1) / TW, (P.H + TH - 1) / TH, P.B);
-  if (out_dtype == DAMVS_F16) warp_agg_h_kernel<C, 8, kAggGwc, __half, DCH, false, MINB, true, G><<<grid, 128, 0, st>>>(P);
-  else warp_agg_h_kernel<C, 8, kAggGwc, __nv_bfloat16, DCH, false, MINB, true, G><<<grid, 128, 0, st>>>(P);
+  if (out_dtype == DAMVS_F16) warp_agg_h_kernel<C, kAggGwc, __half, DCH, MINB, true, G><<<grid, 128, 0, st>>>(P);
+  else warp_agg_h_kernel<C, kAggGwc, __nv_bfloat16, DCH, MINB, true, G><<<grid, 128, 0, st>>>(P);
   DAMVS_LAUNCH_OK("warp_agg_h kernel (group-wise correlation)");
   return DAMVS_OK;
 }
 
 bool warp_gwc_fast_supported(int C, int G, int D, int n_src, int feat_dtype, int out_dtype) {
-  static const bool off = getenv("DAMVS_GWC_PLAIN") != nullptr;   // development knob: A/B against warp_gwc.cu's kernel
   const int dch = C == 32 ? HCfg<32>::DCH : (C == 16 ? HCfg<16>::DCH : HCfg<8>::DCH);
-  return !off && feat_dtype == DAMVS_F16 && (out_dtype == DAMVS_F16 || out_dtype == DAMVS_BF16) && D % dch == 0 && n_src <= kMaxSrcH;
+  return feat_dtype == DAMVS_F16 && (out_dtype == DAMVS_F16 || out_dtype == DAMVS_BF16) && D % dch == 0 && n_src <= kMaxSrcH;
 }
 
 int warp_gwc_fast_launch(const void* ref, const void* const* src, int n_src, const float* rot_trans, const float* hyp, void* out, int B, int C,
