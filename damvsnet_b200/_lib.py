@@ -69,6 +69,10 @@ _SIGNATURES = {
     "damvs_uncertainty_samples_fwd": (c_int, [c_void_p, c_void_p, c_void_p] + [c_int] * 7 + [c_void_p]),
     "damvs_geo_consistency_fuse": (c_int, [c_void_p] * 4 + [POINTER(c_void_p), POINTER(c_double), c_int, c_int, c_int, c_float, c_float, c_float,
                                            c_double, c_double] + [c_void_p] * 5),
+    "damvs_geo_consistency_points_workspace_bytes": (c_size_t, [c_int, c_int]),
+    "damvs_geo_consistency_points": (c_int, [c_void_p] * 4 + [POINTER(c_void_p), POINTER(c_double), POINTER(c_double), c_int, c_int,
+                                             c_int, c_float, c_float, c_float, c_double, c_double, c_void_p, c_longlong]
+                                     + [c_void_p] * 5),
     "damvs_cross_view_terms": (c_int, [c_void_p, c_void_p, POINTER(c_void_p), c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "damvs_cross_view_select": (c_int, [c_void_p, c_void_p, c_int, c_longlong, c_void_p, c_void_p]),
     "damvs_cross_view_bwd": (c_int, [c_void_p, c_void_p, POINTER(c_void_p), c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),

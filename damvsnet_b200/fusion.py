@@ -70,21 +70,62 @@ def backproject_valid(depth: torch.Tensor, mask: torch.Tensor, K, E) -> torch.Te
     return world.t().float()
 
 
+def _enqueue_points(depths, confidences, images, Ks, Es, pairs, conf_thr, dist_base, rel_diff_base):
+    """Enqueue one damvs_geo_consistency_points launch per (ref, srcs) of `pairs`, all appending to one buffer, with
+    no host synchronisation.  Returns (total, xyz, rgb): the device int64 point count and the [capacity,3] buffers,
+    capacity being the number of reference pixels, so that no scan can overflow it."""
+    if not pairs:
+        raise ValueError("pairs is empty")
+    dev = depths[pairs[0][0]].device
+    if dev.type != "cuda":
+        raise ValueError("expected CUDA tensors")
+    views = []
+    for ref, srcs in pairs:
+        if not 1 <= len(srcs) <= MAX_SRC_VIEWS:
+            raise ValueError(f"1..{MAX_SRC_VIEWS} source views supported (the reference's mask list covers dy_range <= 11)")
+        maps = [depths[ref], *confidences[ref], *[depths[s] for s in srcs]]
+        h, w = maps[0].shape
+        if len(confidences[ref]) != 3 or any(t.dtype != torch.float32 or t.device != dev or tuple(t.shape) != (h, w) for t in maps):
+            raise ValueError("expected CUDA fp32 [H,W] maps on one device: depth, three confidences, n source depths")
+        img = images[ref]
+        if img.dtype != torch.float32 or img.device != dev or tuple(img.shape) != (h, w, 3):
+            raise ValueError("expected a CUDA fp32 [H,W,3] image per reference view, on the device of the depth maps")
+        views.append((ref, srcs, [t.contiguous() for t in maps], img.contiguous()))
+    lib = _lib.load()
+    capacity = sum(maps[0].numel() for _, _, maps, _ in views)
+    ws_bytes = [lib.damvs_geo_consistency_points_workspace_bytes(*maps[0].shape) for _, _, maps, _ in views]
+    xyz = torch.empty((capacity, 3), dtype=torch.float32, device=dev)
+    rgb = torch.empty((capacity, 3), dtype=torch.uint8, device=dev)
+    total = torch.zeros((), dtype=torch.int64, device=dev)
+    workspace = torch.zeros(sum(ws_bytes), dtype=torch.uint8, device=dev)   # one zeroed slice per launch
+    offset = 0
+    with torch.cuda.device_of(total):
+        for (ref, srcs, maps, img), nbytes in zip(views, ws_bytes):
+            cams = pack_cameras(Ks[ref], Es[ref], [Ks[s] for s in srcs], [Es[s] for s in srcs])
+            world_from_cam = np.ascontiguousarray(np.linalg.inv(np.asarray(Es[ref], np.float64))[:3])
+            src_ptrs = (ctypes.c_void_p * len(srcs))(*[t.data_ptr() for t in maps[4:]])
+            _lib.check(lib.damvs_geo_consistency_points(
+                _p(maps[0]), _p(maps[1]), _p(maps[2]), _p(maps[3]), src_ptrs, cams.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+                world_from_cam.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), len(srcs), *maps[0].shape,
+                float(conf_thr[0]), float(conf_thr[1]), float(conf_thr[2]), float(dist_base), float(rel_diff_base),
+                _p(img), capacity, _p(xyz), _p(rgb), _p(total), ctypes.c_void_p(workspace.data_ptr() + offset), _stream()))
+            offset += nbytes
+    return total, xyz, rgb
+
+
 def fuse_views(depths: Sequence[torch.Tensor], confidences: Sequence[Sequence[torch.Tensor]], images: Sequence[torch.Tensor],
                Ks, Es, pairs: Sequence[tuple], conf_thr: Sequence[float] = (0.1, 0.15, 0.9), dist_base: float = 1 / 4,
                rel_diff_base: float = 1 / 1300):
     """The loop of reference filter/dypcd.py:filter_depth (:190-300) over a scan that is already on the GPU: for every
     (ref_view, src_views) of `pairs` the fused filter, then the world-space points of the final mask with the reference
     image's colours.  depths[v] [H,W], confidences[v] = (stage1, stage2, stage3) maps, images[v] [H,W,3] in [0,1].
-    Returns (xyz [n,3] fp32, rgb [n,3] uint8) on the device, in the reference's order (views, then row-major pixels)."""
-    xyz, rgb = [], []
-    for ref, srcs in pairs:
-        out = filter_reference_view(depths[ref], confidences[ref], Ks[ref], Es[ref], [depths[s] for s in srcs],
-                                    [Ks[s] for s in srcs], [Es[s] for s in srcs], conf_thr, dist_base, rel_diff_base)
-        m = out["final_mask"]
-        xyz.append(backproject_valid(out["depth_est_averaged"], m, Ks[ref], Es[ref]))
-        rgb.append((images[ref][m] * 255).to(torch.uint8))                       # filter/dypcd.py:299
-    return torch.cat(xyz, 0), torch.cat(rgb, 0)
+    Returns (xyz [n,3] fp32, rgb [n,3] uint8) on the device, in the reference's order (views, then row-major pixels).
+    One native launch per view writes the points straight into a scan-wide buffer; the host waits once, for the count."""
+    total, xyz, rgb = _enqueue_points(depths, confidences, images, Ks, Es, pairs, conf_thr, dist_base, rel_diff_base)
+    n = int(total.item())
+    if n > len(xyz):
+        raise RuntimeError(f"fuse_views: {n} points overflow the buffer of {len(xyz)}")
+    return xyz[:n].clone(), rgb[:n].clone()
 
 
 def write_ply(path: str, xyz, rgb) -> None:

@@ -287,6 +287,27 @@ int damvs_geo_consistency_fuse(const float* depth_ref, const float* conf1, const
                                float conf_thr1, float conf_thr2, float conf_thr3, double dist_base, double rel_diff_base,
                                float* depth_avg, uint8_t* photo_mask, uint8_t* geo_mask, uint8_t* final_mask, void* stream);
 
+/* The same filter, emitting the reference view's share of the scan's point cloud instead of the maps (the
+ * back-projection and colouring of filter_depth, filter/dypcd.py:281-299).  Its masks are those of
+ * damvs_geo_consistency_fuse (one device function computes both).  Inputs as above, plus:
+ *   ref_world_from_cam   HOST float64: inv(E_ref) rows 0-2 [12]
+ *   image                device [H,W,3] fp32 in [0,1]: the reference view's colours
+ *   xyz [capacity,3] fp32, rgb [capacity,3] uint8 out: for every pixel of the final mask, in row-major pixel order,
+ *                        inv(E_ref) [inv(K_ref) [x,y,1] d; 1] (float64, then cast; d the averaged depth) and
+ *                        (uint8)(image * 255) with the product in fp32, truncated
+ *   total                device int64, read and written: the points already in xyz / rgb.  This view's points go to
+ *                        indices total, total + 1, ...; the launch adds its count.  Launches on one stream therefore
+ *                        append view after view without a host synchronisation.
+ *   workspace            device, damvs_geo_consistency_points_workspace_bytes(H, W) bytes, zeroed before each launch
+ * A point whose index is >= capacity is not written but is counted in total, so total > capacity after the launches
+ * means the buffers were too small.  total and workspace are 8-byte aligned; capacity >= 0.                       */
+size_t damvs_geo_consistency_points_workspace_bytes(int H, int W);
+int damvs_geo_consistency_points(const float* depth_ref, const float* conf1, const float* conf2, const float* conf3,
+                                 const float* const* depth_src, const double* cams, const double* ref_world_from_cam,
+                                 int n_src, int H, int W, float conf_thr1, float conf_thr2, float conf_thr3,
+                                 double dist_base, double rel_diff_base, const float* image, long long capacity,
+                                 float* xyz, uint8_t* rgb, long long* total, void* workspace, void* stream);
+
 /* ---- cross-view photometric loss (training-side neighbour of the path) -----------------------------------
  * Fuses cross_view_loss (models/module.py:624-691) and inverse_warping (models/homography.py:7-201) for one stage:
  *   depth_est, depth_gt  device [B,H,W] fp32
